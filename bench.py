@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # our CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    # the reference's own CPU path (unmodified reference staged
                                                            # under oracle/_ref/py + its C++ index_max; else the port)
+  python bench.py ... --dump-outputs DIR                   # also write the outputs of the last timed step to DIR/*.npy
 
 Workload (config.workload): BASELINE.json configs[2] "KITTI detector" -- per rank B=8 pairs = 16 clouds,
 N=16384 points, M=512 nodes, S=4, node kNN K=16, train-mode BatchNorm, probabilistic chamfer + 2x
@@ -313,7 +314,12 @@ def main():
     ap.add_argument("--no-descriptor", action="store_true", help="skip the descriptor-path sub-record (N=1 only)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA-graph replay of the step")
     ap.add_argument("--nbatches", type=int, default=18, help="distinct resident input batches (18 x 7.3 MB > 126 MB L2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed fwd+loss step returned (keypoints, sigmas, nodes, losses; rank 0) as "
+                         "DIR/<name>.npy in float32, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -398,6 +404,8 @@ def main():
         step_resident(i)
     t_load0 = time.time()
     ms, launches = timed(step_resident, K)
+    # copied now: the steps below overwrite the graph's static output tensors
+    outputs = {k: getattr(md, k).detach().float().cpu().numpy() for k in ModelDetector._GRAPH_OUTPUTS} if args.dump_outputs else None
     # the timed region is over (ms is final); the same steps keep the GPU under the same load until the sampler has seen it
     t_load1 = time.time()
     while sampler.count_between(t_load0, t_load1) < 3 and time.time() - t_load0 < 2.0:
@@ -564,6 +572,10 @@ def main():
             line["reference_gpu"] = ref_gpu
         if desc:
             line["descriptor"] = desc
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for k, v in outputs.items():
+                np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
         print(json.dumps(line), flush=True)
     if world > 1:
         # the train-step graph holds the captured NCCL all-reduce: graphs first, then the communicator (usip_b200/dp.py);

@@ -1,11 +1,11 @@
 """-m gpu parity tests of the individual C-ABI kernels against oracle/ (bit-exact for index / integer work,
-1e-4 relative for fp) and, where it travelled, against the reference's own CUDA extensions (oracle/_ref)."""
+1e-4 relative for fp) and against outputs of the reference's own CUDA extensions stored in tests/golden/."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import usip_oracle as orc
-from tests.util_gpu import cu, dev, golden, ref_ext, rel_err
+from tests.util_gpu import cu, dev, digest, golden, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -52,19 +52,20 @@ def test_index_max_bucket_kernel_edge_cases():
     assert np.array_equal(out, orc.index_max(data, index, K))
 
 
-def test_index_max_vs_reference_cuda_full_size():
-    """KITTI shape (B'=16, C=128, N=16384, K=512) against the reference's own kernel (global-mem variant, no cap)."""
-    from usip_b200 import index_max
-    ref = ref_ext("index_max")
-    if ref is None:
-        pytest.skip("oracle/_ref/index_max not built")
+def index_max_full_size_inputs():
     torch.manual_seed(0)
     data = torch.randn(16, 128, 16384, device=dev())
     index = torch.randint(0, 512, (16, 16384), device=dev(), dtype=torch.int32)
+    return data, index
+
+
+def test_index_max_vs_reference_cuda_full_size():
+    """KITTI shape (B'=16, C=128, N=16384, K=512) against the reference's own kernel (global-mem variant, no cap); its
+    output on these inputs is stored as a digest (tools/make_golden_gpu.py)."""
+    from usip_b200 import index_max
+    data, index = index_max_full_size_inputs()
     ours = index_max.forward_cuda_shared_mem(data, index, 512)
-    theirs = ref.forward_cuda(data, index, 512)
-    torch.cuda.synchronize()
-    assert torch.equal(ours, theirs)
+    assert digest(ours) == str(golden("ref_gpu_ops.npz")["index_max_full_size"])
 
 
 def test_index_max_errors():
@@ -91,21 +92,23 @@ def test_ball_query_dist_vs_oracle(B, M, N, K, r):
     assert np.array_equal(out, orc.ball_query_dist(dist, r, K))
 
 
-def test_ball_query_vs_reference_cuda():
-    from usip_b200 import ball_query
-    ref = ref_ext("ball_query")
-    if ref is None:
-        pytest.skip("oracle/_ref/ball_query not built")
+def ball_query_inputs():
     torch.manual_seed(1)
     pc = torch.rand(8, 3, 4096, device=dev()) * 8
     kp = pc[:, :, :256] + 0.05 * torch.randn(8, 3, 256, device=dev())
     dist = torch.norm(kp.unsqueeze(3) - pc.unsqueeze(2), dim=1).contiguous()
+    return pc, kp, dist
+
+
+def test_ball_query_vs_reference_cuda():
+    """Against the reference's own kernel, whose output on these inputs is stored as a digest (tools/make_golden_gpu.py)."""
+    from usip_b200 import ball_query
+    pc, kp, dist = ball_query_inputs()
+    theirs = str(golden("ref_gpu_ops.npz")["ball_query"])
     ours = ball_query.forward_cuda_shared_mem(dist, 1.0, 64)
-    theirs = ref.forward_cuda_shared_mem(dist, 1.0, 64)
-    torch.cuda.synchronize()
-    assert torch.equal(ours, theirs)
+    assert digest(ours) == theirs
     fused, _ = ball_query.forward_fused(pc.contiguous(), None, kp.contiguous(), 1.0, 64, want_group=False)
-    assert torch.equal(fused, theirs)
+    assert digest(fused) == theirs
 
 
 @pytest.mark.parametrize("S", [0, 4])
@@ -320,10 +323,23 @@ def test_pairwise_min_full_size_properties():
 
 def test_ball_group_grid_full_size_vs_reference_cuda():
     """Oxford descriptor shape (B'=16, N=16384, 1024 keypoints, r=1, K=64): cell-binned fused kernel vs the reference
-    kernel on the materialised torch.norm distance matrix (bit-exact indices), plus a dense cloud that exercises the
-    sort path (hits > K) and the in-order fallback (hits > 256)."""
-    from usip_b200 import ball_query
-    ref = ref_ext("ball_query")
+    kernel on the materialised torch.norm distance matrix (bit-exact indices, stored as digests by
+    tools/make_golden_gpu.py), plus a dense cloud that exercises the sort path (hits > K) and the in-order fallback
+    (hits > 256)."""
+    g = golden("ref_gpu_ops.npz")
+    for dense, pc, sn, kp, K in ball_group_grid_cases():
+        B, M = kp.shape[0], kp.shape[2]
+        idx, grp, rows = ops_ball_group(pc, sn, kp, 1.0, K)
+        assert digest(idx) == str(g["ball_group_grid_dense" if dense else "ball_group_grid"]), dense
+        x_aug = torch.cat([pc, sn], 1)
+        gi = idx.long().view(B, 1, M * K).expand(B, 7, M * K)
+        ball = torch.gather(x_aug, 2, gi).view(B, 7, M, K).clone()
+        ball[:, :3] -= kp.unsqueeze(3)
+        assert torch.equal(grp, ball)
+        assert torch.equal(rows.view(B, M, K, 8)[..., :7].permute(0, 3, 1, 2), ball)
+
+
+def ball_group_grid_cases():
     torch.manual_seed(3)
     for dense in (False, True):
         B, N, M, K = (16, 16384, 1024, 64) if not dense else (2, 8192, 256, 64)
@@ -332,20 +348,7 @@ def test_ball_group_grid_full_size_vs_reference_cuda():
         sn = torch.randn(B, 4, N, device=dev())
         sel = torch.randint(0, N, (B, M), device=dev())
         kp = torch.gather(pc, 2, sel.unsqueeze(1).expand(B, 3, M)) + 0.1 * torch.randn(B, 3, M, device=dev())
-        idx, grp, rows = ops_ball_group(pc, sn, kp, 1.0, K)
-        if ref is not None:
-            dist = torch.norm(kp.unsqueeze(3) - pc.unsqueeze(2), dim=1).contiguous()
-            theirs = ref.forward_cuda_shared_mem(dist, 1.0, K)
-            torch.cuda.synchronize()
-            assert torch.equal(idx, theirs), dense
-        else:
-            assert np.array_equal(idx[:2].cpu().numpy(), orc.ball_query_xyz(pc[:2].cpu().numpy(), kp[:2].cpu().numpy(), 1.0, K))
-        x_aug = torch.cat([pc, sn], 1)
-        gi = idx.long().view(B, 1, M * K).expand(B, 7, M * K)
-        ball = torch.gather(x_aug, 2, gi).view(B, 7, M, K).clone()
-        ball[:, :3] -= kp.unsqueeze(3)
-        assert torch.equal(grp, ball)
-        assert torch.equal(rows.view(B, M, K, 8)[..., :7].permute(0, 3, 1, 2), ball)
+        yield dense, pc, sn, kp, K
 
 
 def ops_ball_group(pc, sn, kp, r, K):

@@ -1,5 +1,6 @@
 """Shared helpers for the -m gpu parity tests (the CUDA path is called through the C ABI via usip_b200.ops /
 usip_b200.models; the checker is oracle/ and the reference goldens)."""
+import hashlib
 import os
 import types
 
@@ -49,6 +50,15 @@ def load_params(module, P):
 def golden(name):
     here = os.path.dirname(os.path.abspath(__file__))
     return np.load(os.path.join(here, "golden", name), allow_pickle=False)
+
+
+def digest(t):
+    """SHA-256 over shape, dtype and bytes of a tensor / array: bit-for-bit comparison against a stored output that is
+    too large to keep in tests/golden/."""
+    a = np.ascontiguousarray(t.detach().cpu().numpy() if torch.is_tensor(t) else t)
+    h = hashlib.sha256(repr((a.shape, a.dtype.str)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
 
 
 def ref_ext(name):
