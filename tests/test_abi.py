@@ -65,3 +65,19 @@ def test_product_code_never_imports_oracle():
                 txt = open(os.path.join(dp, f)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, flags=re.M), os.path.join(dp, f)
                 assert "usip_oracle" not in txt or f == "index_max.py", os.path.join(dp, f)
+
+
+def test_only_ops_calls_the_c_abi():
+    """ops.py is the one module that knows the C calling convention: no other Python module of the package calls a usip_*
+    entry point (_lib.py only loads the library and reads its error), and ops.py wraps every launch entry point."""
+    from usip_b200 import _lib
+    pkg = os.path.join(ROOT, "usip_b200")
+    for dp, _, fs in os.walk(pkg):
+        for f in fs:
+            path = os.path.join(dp, f)
+            if f.endswith(".py") and os.path.relpath(path, pkg) not in ("ops.py", "_lib.py"):
+                assert not re.search(r"\busip_[a-z0-9_]+\(", open(path).read()), path
+    ops_src = open(os.path.join(pkg, "ops.py")).read()
+    host_only = ("_abi_version", "_last_error", "_scratch_bytes", "_tile_rows", "_stat_slots", "_tc_workspace_bytes")
+    unwrapped = [n for n in _lib.SIGNATURES if not n.endswith(host_only) and not re.search(r"\b%s\(" % n, ops_src)]
+    assert not unwrapped, unwrapped

@@ -128,8 +128,7 @@ def prepack_weights(module):
     _PACK_STEP[0] = step + 1
     if not jobs:
         return 0
-    arr = (ops.LayerDesc * len(jobs))(*[ent.desc for ent, _ in jobs])
-    ops.check(_lib.load().usip_layer_tc_pack_many(arr, len(jobs), ops._stream()), "usip_layer_tc_pack_many")
+    ops.layer_tc_pack_many([ent.desc for ent, _ in jobs])
     for ent, ver in jobs:
         ent.ver = ver
     return len(jobs)
@@ -144,7 +143,6 @@ def invalidate_packed_weights(module):
         p.__dict__.pop("_usip_tc", None)
 
 
-import os as _os
 _TC_PREC = 1          # usip_layer_desc.precision of the tcgen05 3xTF32 kernel
 
 
@@ -159,12 +157,10 @@ def _precision_for(P, Cin, Cout, use_tc, group=0):
 class LayerRunner:
     """Runs conv1x1(+BN) layers of one nn.Module tree through usip_layer_fwd / usip_bn_finalize."""
 
-    def __init__(self, net, training, use_tc, dev):
-        self.net = net
+    def __init__(self, training, use_tc, dev):
         self.training = training
         self.use_tc = use_tc
         self.dev = dev
-        self.tile = ops.tile_rows()
 
     def bn_state(self, norm, part, ntiles, count, momentum):
         C = norm.weight.numel()
@@ -223,6 +219,13 @@ class LayerRunner:
                 st = self.bn_state(norm, part, ntiles, P if count is None else count, momentum)
         return Y, st, grp
 
+    def run_module(self, m, X, P, epoch=None, **kw):
+        """run() for the conv1x1(+BN) module m: weight, bias and BatchNorm (if m has one) come from m.  Passing the epoch
+        decays the BN momentum (layers.py:62-66); the reference calls some layers without it, and then it never decays."""
+        norm = getattr(m, "norm", None)
+        mom = 0.1 if norm is None else _bn_mom(norm, epoch)
+        return self.run(X, P, _w2d(m.conv.weight), m.conv.bias.detach(), norm, mom, **kw)
+
 
 def _bn_mom(norm, epoch):
     """layers.py:62-66 -- side effect on norm.momentum kept, like the reference."""
@@ -258,51 +261,43 @@ def _knn_head_forward(R, net, AGG, C1, coords, Bp, M, Kn, epoch, keep):
     with _Prof("knn_combine", nbytes=8.0 * G * Cb):
         ops.knn_combine(Z, cmean, knn_i, W5, W5.stride(0), kb[0].conv.bias.detach(), Y5, part5, Bp, M, Kn, Cb)
     bn5 = R.bn_state(kb[0].norm, part5, nt5, G, _bn_mom(kb[0].norm, epoch))
-    prev, Yprev = bn5, Y5
-    saved_before = [(Y5, bn5)]
-    grp_b = None
-    for li in range(1, len(kb)):
+    before = [(kb[0], Y5, bn5)]                      # (module, pre-BN output, BNState) of every layer
+    for li in range(1, len(kb)):                     # only the last layer returns its group max/min
         last = li == len(kb) - 1
-        Yn, bnn, grp = R.run(Yprev, G, _w2d(kb[li].conv.weight), kb[li].conv.bias.detach(), kb[li].norm,
-                             _bn_mom(kb[li].norm, epoch), prev=prev, group=Kn, want_group=last, want_arg=last and keep,
-                             name="knn_b%d" % li)
-        prev, Yprev = bnn, Yn
-        saved_before.append((Yn, bnn))
-        grp_b = grp if last else grp_b
+        Yn, bnn, grp_b = R.run_module(kb[li], before[-1][1], G, epoch, prev=before[-1][2], group=Kn, want_group=last,
+                                      want_arg=last and keep, name="knn_b%d" % li)
+        before.append((kb[li], Yn, bnn))
     # max over K of the activated features (layers.py:433): from group max/min of the raw output
+    _, Yb, bnb = before[-1]
     amax = torch.empty((Q, Cb), dtype=f32, device=dev)
     with _Prof("group_select"):
-        ops.group_select(grp_b["gmax"], grp_b["gmin"], prev.scale, prev.shift, amax, Q, Cb)
+        ops.group_select(grp_b["gmax"], grp_b["gmin"], bnb.scale, bnb.shift, amax, Q, Cb)
     W8 = _w2d(ka[0].conv.weight)
     U, _, _ = R.run(amax, Q, _cols(W8, 0, Cb), None, relu_in=False, name="knn_a0_node")                                    # max half (layers.py:435)
-    Y8, bn8, _ = R.run(Yprev, G, _cols(W8, Cb), ka[0].conv.bias.detach(), ka[0].norm, _bn_mom(ka[0].norm, epoch),
-                       prev=prev, addend=U, add_group=Kn, name="knn_a0")
-    saved_after = [(Y8, bn8)]
-    prevA, YA = bn8, Y8
-    grp_a = None
+    Y8, bn8, _ = R.run(Yb, G, _cols(W8, Cb), ka[0].conv.bias.detach(), ka[0].norm, _bn_mom(ka[0].norm, epoch),
+                       prev=bnb, addend=U, add_group=Kn, name="knn_a0")
+    after = [(ka[0], Y8, bn8)]
     for li in range(1, len(ka)):
         last = li == len(ka) - 1
-        Yn, bnn, grp = R.run(YA, G, _w2d(ka[li].conv.weight), ka[li].conv.bias.detach(), ka[li].norm,
-                             _bn_mom(ka[li].norm, epoch), prev=prevA, group=Kn, want_group=last, want_arg=last and keep,
-                             write_y=(not last) or keep, name="knn_a%d" % li)
-        prevA, YA = bnn, Yn
-        saved_after.append((Yn, bnn))
-        grp_a = grp if last else grp_a
-    ops.group_select(grp_a["gmax"], grp_a["gmin"], prevA.scale, prevA.shift, AGG[:, C1:], Q, C2)   # layers.py:438
+        Yn, bnn, grp_a = R.run_module(ka[li], after[-1][1], G, epoch, prev=after[-1][2], group=Kn, want_group=last,
+                                      want_arg=last and keep, write_y=(not last) or keep, name="knn_a%d" % li)
+        after.append((ka[li], Yn, bnn))
+    bna = after[-1][2]
+    ops.group_select(grp_a["gmax"], grp_a["gmin"], bna.scale, bna.shift, AGG[:, C1:], Q, C2)   # layers.py:438
 
     # ---- head (networks.py:143-154); mlp1/mlp2 are called WITHOUT epoch in the reference
-    Y10, bn10, _ = R.run(AGG, Q, _w2d(net.mlp1.conv.weight), net.mlp1.conv.bias.detach(), net.mlp1.norm,
-                         net.mlp1.norm.momentum, relu_in=False, name="mlp1")
-    Y11, bn11, _ = R.run(Y10, Q, _w2d(net.mlp2.conv.weight), net.mlp2.conv.bias.detach(), net.mlp2.norm,
-                         net.mlp2.norm.momentum, prev=bn10, name="mlp2")
-    OUT, _, _ = R.run(Y11, Q, _w2d(net.mlp3.conv.weight), net.mlp3.conv.bias.detach(), prev=bn11, name="mlp3")
+    Y10, bn10, _ = R.run_module(net.mlp1, AGG, Q, relu_in=False, name="mlp1")
+    Y11, bn11, _ = R.run_module(net.mlp2, Y10, Q, prev=bn10, name="mlp2")
+    OUT, _, _ = R.run_module(net.mlp3, Y11, Q, prev=bn11, name="mlp3")
     with _Prof("head_finalize"):
         keypoints, sigmas = ops.head_finalize(OUT, cmean, opt.loss_sigma_lower_bound, Bp, M)
 
     kctx = dict(knn_i=knn_i)
     if keep:
-        kctx.update(Kn=Kn, C1=C1, C2=C2, Cb=Cb, AGG=AGG, Z=Z, before=saved_before, grp_b=grp_b, amax=amax, U=U,
-                    after=saved_after, grp_a=grp_a, Y10=Y10, bn10=bn10, Y11=Y11, bn11=bn11, OUT=OUT, coords=coords)
+        # head: AGG as the raw input of mlp1, then (module, pre-BN output, BNState) of mlp1..mlp3
+        kctx.update(Kn=Kn, C1=C1, C2=C2, Cb=Cb, AGG=AGG, Z=Z, before=before, grp_b=grp_b, amax=amax, U=U,
+                    after=after, grp_a=grp_a, coords=coords,
+                    head=[(None, AGG, None), (net.mlp1, Y10, bn10), (net.mlp2, Y11, bn11), (net.mlp3, OUT, None)])
     return keypoints, sigmas, kctx
 
 
@@ -324,9 +319,7 @@ def detector_forward(net, x, sn, node, epoch=None, use_tc=True, keep=False):
     S = opt.surface_normal_len if opt.surface_normal_len >= 1 else 0
     Kn = opt.node_knn_k_1
     P, Q = Bp * N, Bp * M
-    G = Q * Kn
-    training = net.training
-    R = LayerRunner(net, training, use_tc, dev)
+    R = LayerRunner(net.training, use_tc, dev)
     x = x.detach().contiguous(); node = node.detach().contiguous()
     snc = sn.detach().contiguous() if S else None
 
@@ -341,9 +334,9 @@ def detector_forward(net, x, sn, node, epoch=None, use_tc=True, keep=False):
     # ---- first PointNet (3+S -> C1/2 -> C1/2 -> C1/2), networks.py:111-114
     fp = net.first_pointnet.layers
     H = fp[0].conv.weight.shape[0]
-    Y0, bn0, _ = R.run(X0, P, _w2d(fp[0].conv.weight), fp[0].conv.bias.detach(), fp[0].norm, _bn_mom(fp[0].norm, epoch), name="pn1.0")
-    Y1, bn1, _ = R.run(Y0, P, _w2d(fp[1].conv.weight), fp[1].conv.bias.detach(), fp[1].norm, _bn_mom(fp[1].norm, epoch), prev=bn0, name="pn1.1")
-    F1, _, _ = R.run(Y1, P, _w2d(fp[2].conv.weight), fp[2].conv.bias.detach(), prev=bn1, name="pn1.2")
+    Y0, bn0, _ = R.run_module(fp[0], X0, P, epoch, name="pn1.0")
+    Y1, bn1, _ = R.run_module(fp[1], Y0, P, epoch, prev=bn0, name="pn1.1")
+    F1, _, _ = R.run_module(fp[2], Y1, P, prev=bn1, name="pn1.2")
     # ---- pool 1 (index_max + gather * mask, networks.py:117-120)
     with _Prof("segmax1", nbytes=4.0 * P * H):
         pool1, arg1 = ops.segmax(F1, H, seg_off, perm, Bp, N, M, want_arg=keep)
@@ -354,7 +347,7 @@ def detector_forward(net, x, sn, node, epoch=None, use_tc=True, keep=False):
     V, _, _ = R.run(pool1, Q, _cols(W3, H), None, relu_in=False, name="pn2.0_node")
     Y3, bn3, _ = R.run(F1, P, _cols(W3, 0, H), sp[0].conv.bias.detach(), sp[0].norm, _bn_mom(sp[0].norm, epoch),
                        relu_in=False, addend=V, add_index=row_seg, name="pn2.0")
-    F2, _, _ = R.run(Y3, P, _w2d(sp[1].conv.weight), sp[1].conv.bias.detach(), prev=bn3, name="pn2.1")
+    F2, _, _ = R.run_module(sp[1], Y3, P, prev=bn3, name="pn2.1")
     # ---- pool 2 -> first C1 columns of the head input (networks.py:130-133,143)
     C2 = net.knnlayer_1.layers_after[-1].conv.weight.shape[0]
     AGG = torch.empty((Q, C1 + C2), dtype=f32, device=dev)
@@ -370,29 +363,16 @@ def detector_forward(net, x, sn, node, epoch=None, use_tc=True, keep=False):
         ctx = dict(kctx)
         ctx.update(Bp=Bp, N=N, M=M, S=S, H=H,
                    seg_off=seg_off, perm=perm, row_seg=row_seg, min_idx=min_idx, count=count, cmean=cmean,
-                   X0=X0, Y0=Y0, bn0=bn0, Y1=Y1, bn1=bn1, F1=F1, pool1=pool1, arg1=arg1, V=V,
+                   X0=X0, pn1=[(fp[0], Y0, bn0), (fp[1], Y1, bn1), (fp[2], F1, None)], pool1=pool1, arg1=arg1, V=V,
                    Y3=Y3, bn3=bn3, F2=F2, arg2=arg2, use_tc=use_tc)
     aux = dict(min_idx=min_idx, count=count, perm=perm, seg_off=seg_off, knn_i=knn_i)
     return cmean, keypoints, sigmas, ctx, aux
 
 
-# ----------------------------------------------------------------------------- losses (forward)
-def chamfer_prob_forward(src, dst, sig_src, sig_dst):
-    """ChamferLoss_Brute sigma branch (losses.py:79-97).  Returns (out3, saved)."""
-    src = src.contiguous(); dst = dst.contiguous()
-    d_sd, i_sd = ops.pairwise_min(src, dst)
-    d_ds, i_ds = ops.pairwise_min(dst, src)
-    out3 = ops.chamfer_prob_reduce(d_sd, i_sd, d_ds, i_ds, sig_src.contiguous(), sig_dst.contiguous())
-    return out3, (d_sd, i_sd, d_ds, i_ds)
-
-
 class _Bwd:
-    """Small helper bundle for the backward plans: raw C-ABI calls + gradient bookkeeping."""
+    """Gradient bookkeeping of the backward plans and the per-layer steps they are written in."""
 
     def __init__(self, net, dev, use_tc):
-        from . import _lib
-        self.lib = _lib.load()
-        self.check = _lib.check
         self.dev = dev
         self.use_tc = use_tc
         # opt.backward_precision: "3xtf32" (default, fp32-equivalent like the forward) or "tf32" -- the dgrad / wgrad GEMMs as
@@ -422,64 +402,40 @@ class _Bwd:
         g = self.grads[w]
         return g.view(g.shape[0], -1)
 
-    def bn_bwd(self, G, Y, st, norm, P, C, relu=True, name="bn_bwd"):
-        """g_y of a train-mode BN(+ReLU) layer; writes g_gamma / g_beta; returns GY [P,C] (new buffer)."""
-        nt = (P + 127) // 128
-        part = torch.empty((nt, 2, C), dtype=f32, device=self.dev)
-        c1 = torch.empty(C, dtype=f32, device=self.dev); c2 = torch.empty(C, dtype=f32, device=self.dev)
-        GY = torch.empty((P, C), dtype=f32, device=self.dev)
-        s = ops._stream(); p = ops._p
+    def bn_bwd(self, G, Y, st, norm, name="bn_bwd"):
+        """g_y [P,C] (new buffer) of a train-mode BN+ReLU layer from the gradient G of its output; writes g_gamma / g_beta."""
+        P, C = G.shape
         with _Prof(name, nbytes=4.0 * P * C * 5):
-            self.check(self.lib.usip_bn_bwd_reduce(p(G), G.stride(0), p(Y), Y.stride(0), p(st.scale), p(st.shift), p(st.mean),
-                                                   p(st.invstd), 1 if relu else 0, p(part), P, C, s), "usip_bn_bwd_reduce")
-            self.check(self.lib.usip_bn_bwd_finalize(p(part), nt, P, C, p(self.grads[norm.weight]), p(self.grads[norm.bias]),
-                                                     p(c1), p(c2), 1, s), "usip_bn_bwd_finalize")
-            self.check(self.lib.usip_bn_bwd_apply(p(G), G.stride(0), p(Y), Y.stride(0), p(st.scale), p(st.shift), p(st.mean),
-                                                  p(st.invstd), p(c1), p(c2), 1 if relu else 0, p(GY), GY.stride(0), P, C, s),
-                       "usip_bn_bwd_apply")
-        return GY
+            part = ops.bn_bwd_reduce(G, Y, st.scale, st.shift, st.mean, st.invstd, True)
+            c1, c2 = ops.bn_bwd_finalize(part, P, self.grads[norm.weight], self.grads[norm.bias])
+            return ops.bn_bwd_apply(G, Y, st.scale, st.shift, st.mean, st.invstd, c1, c2, True)
 
-    def groupmax_select(self, Gout, grp, st, Qn, C, with_stats):
-        """Gradient of out = max_k relu(bn(y_k)) at the selected row of each group: gz [Qn,C] (ReLU-masked), argsel [Qn,C]
-        and, with_stats, the BN-backward partial sums over the selected entries."""
-        p, s = ops._p, ops._stream
-        gz = torch.empty((Qn, C), dtype=f32, device=self.dev)
-        argsel = torch.empty((Qn, C), dtype=i32, device=self.dev)
-        nt = (Qn + 127) // 128
-        part = torch.empty((nt, 2, C), dtype=f32, device=self.dev) if with_stats else None
-        self.check(self.lib.usip_groupmax_bwd_select(p(Gout), Gout.stride(0), p(grp["gmax"]), p(grp["gmin"]), p(grp["amax"]),
-                                                     p(grp["amin"]), p(st.scale), p(st.shift), p(st.mean), p(st.invstd), p(gz),
-                                                     p(argsel), p(part), Qn, C, s()), "usip_groupmax_bwd_select")
-        return gz, argsel, part, nt
+    def groupmax_select(self, Gout, grp, st, with_stats):
+        """ops.groupmax_bwd_select of out = max_k relu(bn(y_k)) for the group outputs `grp` of LayerRunner.run."""
+        return ops.groupmax_bwd_select(Gout, grp["gmax"], grp["gmin"], grp["amax"], grp["amin"], st.scale, st.shift, st.mean,
+                                       st.invstd, with_stats)
 
-    def groupmax_bn_bwd(self, Gout, Y, grp, st, norm, K, Q, C):
+    def groupmax_bn_bwd(self, Gout, Y, grp, st, norm, K):
         """g_y [Q*K, C] of a layer whose ONLY consumer is max_k relu(bn(y)) (layers.py:433,438; networks.py:572,700)."""
-        p, s = ops._p, ops._stream
-        G = Q * K
-        gz, arg, part, nt = self.groupmax_select(Gout, grp, st, Q, C, True)
-        c1 = torch.empty(C, dtype=f32, device=self.dev); c2 = torch.empty(C, dtype=f32, device=self.dev)
-        self.check(self.lib.usip_bn_bwd_finalize(p(part), nt, G, C, p(self.grads[norm.weight]), p(self.grads[norm.bias]),
-                                                 p(c1), p(c2), 1, s()), "usip_bn_bwd_finalize")
-        GY = torch.empty((G, C), dtype=f32, device=self.dev)
+        G, C = Gout.shape[0] * K, Gout.shape[1]
+        gz, arg, part = self.groupmax_select(Gout, grp, st, True)
+        c1, c2 = ops.bn_bwd_finalize(part, G, self.grads[norm.weight], self.grads[norm.bias])
         with _Prof("groupmax_bwd_apply", nbytes=8.0 * G * C):
-            self.check(self.lib.usip_groupmax_bwd_apply(p(Y), Y.stride(0), p(gz), p(arg), p(st.scale), p(st.mean), p(st.invstd),
-                                                        p(c1), p(c2), p(GY), GY.stride(0), K, G, C, s()), "usip_groupmax_bwd_apply")
-        return GY
+            return ops.groupmax_bwd_apply(Y, gz, arg, st.scale, st.mean, st.invstd, c1, c2, K)
 
-    def wgrad(self, GY, X, gW, P, Cout, Cin, prev=None, relu=False, name="wgrad"):
-        s = ops._stream(); p = ops._p
+    def wgrad(self, GY, X, gW, prev=None, name="wgrad"):
+        """gW += GY^T act(X), act = the BN+ReLU of `prev` (BNState) or the identity."""
+        P, (Cout, Cin) = GY.shape[0], gW.shape
         tc = self.use_tc and Cout % 4 == 0 and Cout >= 64 and Cin % 64 == 0 and P >= 4096
         with _Prof("%s[%dx%d->%d]" % (name, P, Cin, Cout), flops=2.0 * P * Cin * Cout,
                    precision="3xTF32 tcgen05" if tc else "fp32 SIMT"):
-            self.check(self.lib.usip_wgrad(p(GY), GY.stride(0), p(X), X.stride(0), None if prev is None else p(prev.scale),
-                                           None if prev is None else p(prev.shift), 1 if (relu or prev is not None) else 0,
-                                           p(gW), gW.stride(0), P, Cout, Cin, (4 if self.tf32_bwd else 1) if self.use_tc else 0, s), "usip_wgrad")
+            ops.wgrad(GY, X, gW, None if prev is None else prev.scale, None if prev is None else prev.shift, prev is not None,
+                      (4 if self.tf32_bwd else 1) if self.use_tc else 0)
 
-    def dgrad(self, GY, W2d, P, name="dgrad", out=None):
+    def dgrad(self, GY, W2d, name="dgrad"):
         """G_in[P,Cin] = GY[P,Cout] @ W2d[Cout,Cin] (the forward weight, used transposed by the layer kernel)."""
-        Cout, Cin = W2d.shape
-        if out is None:
-            out = torch.empty((P, Cin), dtype=f32, device=self.dev)
+        P, (Cout, Cin) = GY.shape[0], W2d.shape
+        out = torch.empty((P, Cin), dtype=f32, device=self.dev)
         prec = _precision_for(P, Cout, Cin, self.use_tc)
         ws, packed, pack_ent = _tc_workspace(W2d, P, Cout, Cin, 0, True, prec) if prec else (None, False, None)
         with _Prof("%s[%dx%d->%d]" % (name, P, Cout, Cin), flops=2.0 * P * Cin * Cout,
@@ -488,8 +444,20 @@ class _Bwd:
                           debug_flags=8 if (self.tf32_bwd and prec) else 0, pack_entry=pack_ent)
         return out
 
-    def colsum(self, G, out, P, C):
-        self.check(self.lib.usip_colsum(ops._p(G), G.stride(0), ops._p(out), P, C, ops._stream()), "usip_colsum")
+    def layer_bwd(self, GY, m, src, name, bn_name):
+        """Backward of the conv1x1 layer m from GY, the gradient of its pre-BN output rows.  Accumulates m's weight gradient
+        (and its bias gradient when no BN follows m: a bias in front of a train-mode BN has exactly zero gradient) and
+        returns the gradient of what m read.  src = (module, Y, BNState) of the layer m reads through BN+ReLU: the result is
+        the gradient of that layer's pre-BN output Y.  src = (None, X, None): X is m's raw input and the result its gradient."""
+        pm, X, st = src
+        W = _w2d(m.conv.weight)
+        self.wgrad(GY, X, self.g2d(m.conv.weight), prev=st, name="wgrad_" + name)
+        if getattr(m, "norm", None) is None:
+            ops.colsum(GY, self.grads[m.conv.bias])
+        G_in = self.dgrad(GY, W, name="dgrad_" + name)
+        if st is None:
+            return G_in
+        return self.bn_bwd(G_in, X, st, pm.norm, name=bn_name)
 
 
 def _knn_head_backward(bw, net, ctx, g_kp, g_sig):
@@ -497,81 +465,49 @@ def _knn_head_backward(bw, net, ctx, g_kp, g_sig):
     the gradient [Q, C1] of the per-node feature that entered AGG[:, :C1] (head path + kNN path)."""
     dev = bw.dev
     Bp, M = ctx["Bp"], ctx["M"]
-    Kn, C1, C2, Cb = ctx["Kn"], ctx["C1"], ctx["C2"], ctx["Cb"]
+    Kn, C1, Cb = ctx["Kn"], ctx["C1"], ctx["Cb"]
     Q = Bp * M
-    G = Q * Kn
-    lib, check, p, s = bw.lib, bw.check, ops._p, ops._stream
-    kb, ka = net.knnlayer_1.layers_before, net.knnlayer_1.layers_after
+    before, after, head = ctx["before"], ctx["after"], ctx["head"]
     g_kp = None if g_kp is None else g_kp.contiguous()
     g_sig = None if g_sig is None else g_sig.contiguous()
-    # ---- head (networks.py:143-154)
-    G_OUT = torch.empty((Q, 4), dtype=f32, device=dev)
-    check(lib.usip_head_bwd(p(g_kp), p(g_sig), p(ctx["OUT"]), ctx["OUT"].stride(0), p(G_OUT), Bp, M, s()), "usip_head_bwd")
-    W12 = _w2d(net.mlp3.conv.weight)
-    bw.wgrad(G_OUT, ctx["Y11"], bw.g2d(net.mlp3.conv.weight), Q, 4, W12.shape[1], prev=ctx["bn11"], name="wgrad_mlp3")
-    bw.colsum(G_OUT, bw.grads[net.mlp3.conv.bias], Q, 4)
-    G_a11 = bw.dgrad(G_OUT, W12, Q, name="dgrad_mlp3")
-    GY11 = bw.bn_bwd(G_a11, ctx["Y11"], ctx["bn11"], net.mlp2.norm, Q, G_a11.shape[1])
-    W11 = _w2d(net.mlp2.conv.weight)
-    bw.wgrad(GY11, ctx["Y10"], bw.g2d(net.mlp2.conv.weight), Q, W11.shape[0], W11.shape[1], prev=ctx["bn10"], name="wgrad_mlp2")
-    G_a10 = bw.dgrad(GY11, W11, Q, name="dgrad_mlp2")
-    GY10 = bw.bn_bwd(G_a10, ctx["Y10"], ctx["bn10"], net.mlp1.norm, Q, G_a10.shape[1])
-    W10 = _w2d(net.mlp1.conv.weight)
-    bw.wgrad(GY10, ctx["AGG"], bw.g2d(net.mlp1.conv.weight), Q, W10.shape[0], W10.shape[1], name="wgrad_mlp1")
-    G_AGG = bw.dgrad(GY10, W10, Q, name="dgrad_mlp1")                      # [Q, C1+C2]
-    G_pool2 = G_AGG[:, :C1]
-    G_feat = G_AGG[:, C1:]
+    # ---- head (networks.py:143-154): mlp3 -> mlp2 -> mlp1
+    GY = ops.head_bwd(g_kp, g_sig, head[-1][1], Bp, M)
+    for li in range(len(head) - 1, 0, -1):
+        GY = bw.layer_bwd(GY, head[li][0], head[li - 1], "mlp%d" % li, "bn_bwd")
+    G_pool2, G_feat = GY[:, :C1], GY[:, C1:]                               # GY: gradient of AGG [Q, C1+C2]
 
-    # ---- kNN fusion, layers_after (layers.py:435-438)
-    groupmax_select = bw.groupmax_select
-    Ya_last, bna_last = ctx["after"][-1]
-    GYa = bw.groupmax_bn_bwd(G_feat, Ya_last, ctx["grp_a"], bna_last, ka[-1].norm, Kn, Q, C2)
-    # remaining after-layers, last -> first (li >= 1: plain BN+ReLU chains)
-    for li in range(len(ka) - 1, 0, -1):
-        Wl = _w2d(ka[li].conv.weight)
-        Yin, bnin = ctx["after"][li - 1]
-        bw.wgrad(GYa, Yin, bw.g2d(ka[li].conv.weight), G, Wl.shape[0], Wl.shape[1], prev=bnin, name="wgrad_knn_a%d" % li)
-        G_in = bw.dgrad(GYa, Wl, G, name="dgrad_knn_a%d" % li)
-        GYa = bw.bn_bwd(G_in, Yin, bnin, ka[li - 1].norm, G, G_in.shape[1], name="bn_bwd_knn_a%d" % (li - 1))
-        del G_in
+    # ---- kNN fusion, layers_after (layers.py:435-438), last -> 1
+    ka_last, Ya_last, bna_last = after[-1]
+    GYa = bw.groupmax_bn_bwd(G_feat, Ya_last, ctx["grp_a"], bna_last, ka_last.norm, Kn)
+    for li in range(len(after) - 1, 0, -1):
+        GYa = bw.layer_bwd(GYa, after[li][0], after[li - 1], "knn_a%d" % li, "bn_bwd_knn_a%d" % (li - 1))
     # ka[0]: Y8 = a7 Wnb^T + U[row/K] + b, U = amax Wmax^T
-    W8 = _w2d(ka[0].conv.weight)
-    Yb_last, bnb_last = ctx["before"][-1]
-    gW8 = bw.g2d(ka[0].conv.weight)
-    bw.wgrad(GYa, Yb_last, gW8[:, Cb:], G, C2, Cb, prev=bnb_last, name="wgrad_knn_a0")
-    G_a7 = bw.dgrad(GYa, _cols(W8, Cb), G, name="dgrad_knn_a0")               # [G, Cb]
-    G_U = torch.empty((Q, C2), dtype=f32, device=dev)
-    check(lib.usip_group_sum(p(GYa), GYa.stride(0), p(G_U), G_U.stride(0), Kn, Q, C2, s()), "usip_group_sum")
+    ka0, kb0 = after[0][0], before[0][0]
+    W8, gW8 = _w2d(ka0.conv.weight), bw.g2d(ka0.conv.weight)
+    kb_last, Yb_last, bnb_last = before[-1]
+    bw.wgrad(GYa, Yb_last, gW8[:, Cb:], prev=bnb_last, name="wgrad_knn_a0")
+    G_a7 = bw.dgrad(GYa, _cols(W8, Cb), name="dgrad_knn_a0")                 # [G, Cb]
+    G_U = ops.group_sum(GYa, Kn)                                            # [Q, C2]
     del GYa
-    bw.wgrad(G_U, ctx["amax"], gW8[:, :Cb], Q, C2, Cb, name="wgrad_knn_a0_node")
-    G_amax = bw.dgrad(G_U, _cols(W8, 0, Cb), Q, name="dgrad_knn_a0_node")        # [Q, Cb]
+    bw.wgrad(G_U, ctx["amax"], gW8[:, :Cb], name="wgrad_knn_a0_node")
+    G_amax = bw.dgrad(G_U, _cols(W8, 0, Cb), name="dgrad_knn_a0_node")        # [Q, Cb]
     # max path joins the dense gradient of a7 at the arg rows (ReLU mask is applied by bn_bwd below)
-    _, arg7, _, _ = groupmax_select(G_amax, ctx["grp_b"], bnb_last, Q, Cb, False)
-    check(lib.usip_groupmax_scatter_add(p(G_a7), G_a7.stride(0), p(G_amax), p(arg7), Kn, Q, Cb, s()), "usip_groupmax_scatter_add")
+    _, arg7, _ = bw.groupmax_select(G_amax, ctx["grp_b"], bnb_last, False)
+    ops.groupmax_scatter_add(G_a7, G_amax, arg7, Kn)
     # ---- layers_before, last -> 1
-    GYb = bw.bn_bwd(G_a7, Yb_last, bnb_last, kb[-1].norm, G, Cb, name="bn_bwd_knn_b%d" % (len(kb) - 1))
+    GYb = bw.bn_bwd(G_a7, Yb_last, bnb_last, kb_last.norm, name="bn_bwd_knn_b%d" % (len(before) - 1))
     del G_a7
-    for li in range(len(kb) - 1, 0, -1):
-        Wl = _w2d(kb[li].conv.weight)
-        Yin, bnin = ctx["before"][li - 1]
-        bw.wgrad(GYb, Yin, bw.g2d(kb[li].conv.weight), G, Wl.shape[0], Wl.shape[1], prev=bnin, name="wgrad_knn_b%d" % li)
-        G_in = bw.dgrad(GYb, Wl, G, name="dgrad_knn_b%d" % li)
-        GYb = bw.bn_bwd(G_in, Yin, bnin, kb[li - 1].norm, G, G_in.shape[1], name="bn_bwd_knn_b%d" % (li - 1))
-        del G_in
+    for li in range(len(before) - 1, 0, -1):
+        GYb = bw.layer_bwd(GYb, before[li][0], before[li - 1], "knn_b%d" % li, "bn_bwd_knn_b%d" % (li - 1))
     # kb[0] = knn_combine: Y5 = Z[nbr] + Wxyz*delta + b, Z = pool2 Wf^T
-    W5 = _w2d(kb[0].conv.weight)
-    gW5 = bw.g2d(kb[0].conv.weight)
+    W5, gW5 = _w2d(kb0.conv.weight), bw.g2d(kb0.conv.weight)
     G_Z = torch.zeros((Q, Cb), dtype=f32, device=dev)
     with _Prof("knn_combine_bwd"):
-        check(lib.usip_knn_combine_bwd(p(GYb), GYb.stride(0), p(ctx["coords"]), p(ctx["knn_i"]), p(G_Z), G_Z.stride(0), p(gW5),
-                                       gW5.stride(0), Bp, M, Kn, Cb, s()), "usip_knn_combine_bwd")
+        ops.knn_combine_bwd(GYb, ctx["coords"], ctx["knn_i"], G_Z, gW5, Bp, M, Kn)
     del GYb
-    pool2 = ctx["AGG"][:, :C1]
-    bw.wgrad(G_Z, pool2, gW5[:, 3:], Q, Cb, C1, name="wgrad_knn_b0_node")
-    G_pool2_knn = bw.dgrad(G_Z, _cols(W5, 3), Q, name="dgrad_knn_b0_node")    # [Q, C1]
-    G_pool2_tot = G_pool2_knn
+    bw.wgrad(G_Z, ctx["AGG"][:, :C1], gW5[:, 3:], name="wgrad_knn_b0_node")
+    G_pool2_tot = bw.dgrad(G_Z, _cols(W5, 3), name="dgrad_knn_b0_node")       # [Q, C1]
     G_pool2_tot += G_pool2                                                 # tiny [Q,C1] plumbing add
-
     return G_pool2_tot
 
 
@@ -580,51 +516,32 @@ def detector_backward(net, ctx, g_kp, g_sig):
     dev = ctx["cmean"].device
     Bp, N, M = ctx["Bp"], ctx["N"], ctx["M"]
     H, C1 = ctx["H"], ctx["C1"]
-    P, Q = Bp * N, Bp * M
+    P = Bp * N
     bw = _Bwd(net, dev, ctx["use_tc"])
-    lib, check, p, s = bw.lib, bw.check, ops._p, ops._stream
-    fp, sp = net.first_pointnet.layers, net.second_pointnet.layers
+    sp, pn1 = net.second_pointnet.layers, ctx["pn1"]
 
     G_pool2_tot = _knn_head_backward(bw, net, ctx, g_kp, g_sig)
 
     # ---- pool 2 un-pool (index_max gather backward), second PointNet
     G_F2 = torch.zeros((P, C1), dtype=f32, device=dev)
-    check(lib.usip_unpool_scatter(p(G_F2), G_F2.stride(0), p(G_pool2_tot), G_pool2_tot.stride(0), p(ctx["arg2"]), Q, C1, 0, s()),
-          "usip_unpool_scatter")
-    W4 = _w2d(sp[1].conv.weight)
-    bw.wgrad(G_F2, ctx["Y3"], bw.g2d(sp[1].conv.weight), P, C1, C1, prev=ctx["bn3"], name="wgrad_pn2.1")
-    bw.colsum(G_F2, bw.grads[sp[1].conv.bias], P, C1)
-    G_a3 = bw.dgrad(G_F2, W4, P, name="dgrad_pn2.1")
+    ops.unpool_scatter(G_F2, G_pool2_tot, ctx["arg2"], accumulate=False)
+    GY3 = bw.layer_bwd(G_F2, sp[1], (sp[0], ctx["Y3"], ctx["bn3"]), "pn2.1", "bn_bwd_pn2.0")
     del G_F2
-    GY3 = bw.bn_bwd(G_a3, ctx["Y3"], ctx["bn3"], sp[0].norm, P, C1, name="bn_bwd_pn2.0")
-    del G_a3
     W3 = _w2d(sp[0].conv.weight)
     gW3 = bw.g2d(sp[0].conv.weight)
-    bw.wgrad(GY3, ctx["F1"], gW3[:, :H], P, C1, H, name="wgrad_pn2.0")
-    G_F1 = bw.dgrad(GY3, _cols(W3, 0, H), P, name="dgrad_pn2.0")                  # [P, H]
-    G_V = torch.empty((Q, C1), dtype=f32, device=dev)
-    check(lib.usip_seg_sum(p(GY3), GY3.stride(0), p(ctx["seg_off"]), p(G_V), G_V.stride(0), Bp, N, M, C1, s()), "usip_seg_sum")
+    bw.wgrad(GY3, pn1[-1][1], gW3[:, :H], name="wgrad_pn2.0")
+    G_F1 = bw.dgrad(GY3, _cols(W3, 0, H), name="dgrad_pn2.0")                  # [P, H]
+    G_V = ops.seg_sum(GY3, ctx["seg_off"], Bp, N, M)                         # [Q, C1]
     del GY3
-    bw.wgrad(G_V, ctx["pool1"], gW3[:, H:], Q, C1, H, name="wgrad_pn2.0_node")
-    G_pool1 = bw.dgrad(G_V, _cols(W3, H), Q, name="dgrad_pn2.0_node")          # [Q, H]
-    check(lib.usip_unpool_scatter(p(G_F1), G_F1.stride(0), p(G_pool1), G_pool1.stride(0), p(ctx["arg1"]), Q, H, 1, s()),
-          "usip_unpool_scatter")
-    # ---- first PointNet
-    W2 = _w2d(fp[2].conv.weight)
-    bw.wgrad(G_F1, ctx["Y1"], bw.g2d(fp[2].conv.weight), P, H, H, prev=ctx["bn1"], name="wgrad_pn1.2")
-    bw.colsum(G_F1, bw.grads[fp[2].conv.bias], P, H)
-    G_a1 = bw.dgrad(G_F1, W2, P, name="dgrad_pn1.2")
+    bw.wgrad(G_V, ctx["pool1"], gW3[:, H:], name="wgrad_pn2.0_node")
+    G_pool1 = bw.dgrad(G_V, _cols(W3, H), name="dgrad_pn2.0_node")             # [Q, H]
+    ops.unpool_scatter(G_F1, G_pool1, ctx["arg1"], accumulate=True)
+    # ---- first PointNet, last -> 1, then the weight gradient of layer 0 (the points carry none)
+    GY = G_F1
     del G_F1
-    GY1 = bw.bn_bwd(G_a1, ctx["Y1"], ctx["bn1"], fp[1].norm, P, H, name="bn_bwd_pn1.1")
-    del G_a1
-    W1 = _w2d(fp[1].conv.weight)
-    bw.wgrad(GY1, ctx["Y0"], bw.g2d(fp[1].conv.weight), P, H, H, prev=ctx["bn0"], name="wgrad_pn1.1")
-    G_a0 = bw.dgrad(GY1, W1, P, name="dgrad_pn1.1")
-    del GY1
-    GY0 = bw.bn_bwd(G_a0, ctx["Y0"], ctx["bn0"], fp[0].norm, P, H, name="bn_bwd_pn1.0")
-    del G_a0
-    W0 = _w2d(fp[0].conv.weight)
-    bw.wgrad(GY0, ctx["X0"], bw.g2d(fp[0].conv.weight), P, H, W0.shape[1], name="wgrad_pn1.0")
+    for li in range(len(pn1) - 1, 0, -1):
+        GY = bw.layer_bwd(GY, pn1[li][0], pn1[li - 1], "pn1.%d" % li, "bn_bwd_pn1.%d" % (li - 1))
+    bw.wgrad(GY, ctx["X0"], bw.g2d(pn1[0][0].conv.weight), name="wgrad_pn1.0")
     # conv biases in front of a train-mode BatchNorm receive exactly zero gradient (BN removes the mean); they
     # stay zero-initialised in bw.grads.
     return bw.result(net)
@@ -641,21 +558,18 @@ def _group_net_forward(R, net, rows, Bp, M, K, keep, out=None):
     G, Q = Bp * M * K, Bp * M
     c1, c2, c3, c4, c5 = net.conv1, net.conv2, net.conv3, net.conv4, net.conv5
     D = c3.conv.weight.shape[0]
-    Y1, bn1, _ = R.run(rows, G, _w2d(c1.conv.weight), c1.conv.bias.detach(), c1.norm, c1.norm.momentum, name="grp.conv1")
-    Y2, bn2, _ = R.run(Y1, G, _w2d(c2.conv.weight), c2.conv.bias.detach(), c2.norm, c2.norm.momentum, prev=bn1, name="grp.conv2")
-    Y3, bn3, grp3 = R.run(Y2, G, _w2d(c3.conv.weight), c3.conv.bias.detach(), c3.norm, c3.norm.momentum, prev=bn2,
-                          group=K, want_group=True, want_arg=keep, name="grp.conv3")
+    Y1, bn1, _ = R.run_module(c1, rows, G, name="grp.conv1")
+    Y2, bn2, _ = R.run_module(c2, Y1, G, prev=bn1, name="grp.conv2")
+    Y3, bn3, grp3 = R.run_module(c3, Y2, G, prev=bn2, group=K, want_group=True, want_arg=keep, name="grp.conv3")
     amax = torch.empty((Q, D), dtype=f32, device=dev)
     ops.group_select(grp3["gmax"], grp3["gmin"], bn3.scale, bn3.shift, amax, Q, D)          # y_first_max (networks.py:377)
     W4 = _w2d(c4.conv.weight)
-    C4 = W4.shape[0]
     U, _, _ = R.run(amax, Q, _cols(W4, D), None, relu_in=False, name="grp.conv4_node")        # cat(y_first, max): max is LAST
     Y4, bn4, _ = R.run(Y3, G, _cols(W4, 0, D), c4.conv.bias.detach(), c4.norm, c4.norm.momentum, prev=bn3, addend=U,
                        add_group=K, name="grp.conv4")
     last_bn = getattr(c5, "norm", None) is not None
-    Y5, bn5, grp5 = R.run(Y4, G, _w2d(c5.conv.weight), c5.conv.bias.detach(), c5.norm if last_bn else None,
-                          c5.norm.momentum if last_bn else 0.1, prev=bn4, group=K, want_group=True, want_arg=keep,
-                          write_y=last_bn and keep, name="grp.conv5")
+    Y5, bn5, grp5 = R.run_module(c5, Y4, G, prev=bn4, group=K, want_group=True, want_arg=keep, write_y=last_bn and keep,
+                                 name="grp.conv5")
     result = grp5["gmax"]
     if last_bn:
         C5 = c5.conv.weight.shape[0]
@@ -665,8 +579,8 @@ def _group_net_forward(R, net, rows, Bp, M, K, keep, out=None):
         result = out
     gctx = dict(D=D)
     if keep:
-        gctx.update(Bp=Bp, M=M, K=K, C4=C4, rows=rows, Y1=Y1, bn1=bn1, Y2=Y2, bn2=bn2, Y3=Y3, bn3=bn3, grp3=grp3, amax=amax,
-                    Y4=Y4, bn4=bn4, Y5=Y5, bn5=bn5, grp5=grp5)
+        gctx.update(Bp=Bp, M=M, K=K, rows=rows, layers=[(c1, Y1, bn1), (c2, Y2, bn2), (c3, Y3, bn3), (c4, Y4, bn4)],
+                    grp3=grp3, amax=amax, Y5=Y5, bn5=bn5, grp5=grp5)
     return result, gctx
 
 
@@ -690,7 +604,7 @@ def ablation_forward(net, x, sn, node, epoch=None, use_tc=True, keep=False, mode
     Kn = opt.node_knn_k_1
     K = ABLATION_K
     Q = Bp * M
-    R = LayerRunner(net, net.training, use_tc, dev)
+    R = LayerRunner(net.training, use_tc, dev)
     x = x.detach().contiguous(); node = node.detach().contiguous()
     snc = sn.detach().contiguous() if S else None
     with _Prof("group_%s" % mode):
@@ -714,11 +628,9 @@ def ablation_backward(net, ctx, g_kp, g_sig):
     """Backward of ablation_forward: gradients of net.parameters() in order (points and nodes carry none)."""
     dev = ctx["AGG"].device
     gctx = ctx["group_net"]
-    Bp, M, K = ctx["Bp"], ctx["M"], gctx["K"]
     bw = _Bwd(net, dev, ctx["use_tc"])
     G_pool = _knn_head_backward(bw, net, ctx, g_kp, g_sig)                  # gradient of max_k relu(bn5(conv5)) [Q, C1]
-    C5 = net.conv5.conv.weight.shape[0]
-    GY5 = bw.groupmax_bn_bwd(G_pool, gctx["Y5"], gctx["grp5"], gctx["bn5"], net.conv5.norm, K, Bp * M, C5)
+    GY5 = bw.groupmax_bn_bwd(G_pool, gctx["Y5"], gctx["grp5"], gctx["bn5"], net.conv5.norm, gctx["K"])
     _group_net_backward(bw, net, gctx, GY5)
     return bw.result(net)
 
@@ -726,7 +638,6 @@ def ablation_backward(net, ctx, g_kp, g_sig):
 def descriptor_forward(net, x, sn, keypoints, epoch, permute_idx, use_tc=True, keep=False):
     """DescriptorLiteOld.forward (models/networks.py:333-385) on the fused plan.
     Returns (descriptor (B,C,M), x_features (B,3+S,M,K), ctx) -- ctx holds what descriptor_backward needs (keep=True)."""
-    from . import _lib
     opt = net.opt
     dev = x.device
     if keep and not net.training:
@@ -736,8 +647,7 @@ def descriptor_forward(net, x, sn, keypoints, epoch, permute_idx, use_tc=True, k
     M = keypoints.shape[2]
     K = opt.ball_nsamples
     S = opt.surface_normal_len if opt.surface_normal_len > 0 else 0
-    G, Q = Bp * M * K, Bp * M
-    R = LayerRunner(net, net.training, use_tc, dev)
+    R = LayerRunner(net.training, use_tc, dev)
     # permute the points on the host-drawn permutation: the ball query keeps the FIRST K hits in index order
     x = x.detach()[:, :, permute_idx].contiguous()
     snp = sn.detach()[:, :, permute_idx].contiguous() if S else None
@@ -745,10 +655,7 @@ def descriptor_forward(net, x, sn, keypoints, epoch, permute_idx, use_tc=True, k
     with _Prof("ball_group", nbytes=4.0 * Bp * (N * (3 + S) + 3 * M + M * K + (3 + S) * M * K)):
         idx, feats, rows = ops.ball_group(x, snp, kp, float(opt.ball_radius), K, want_group=True, rows_ld=8)
     gmax5, gctx = _group_net_forward(R, net, rows, Bp, M, K, keep, out=None)
-    D = gctx["D"]
-    desc = torch.empty((Bp, D, M), dtype=f32, device=dev)
-    _lib.check(_lib.load().usip_l2norm_to_bcm(ops._p(gmax5), gmax5.stride(0), ops._p(desc), None, Bp, M, D,
-                                              ops._stream()), "usip_l2norm_to_bcm")
+    desc = ops.l2norm_to_bcm(gmax5, Bp, M)
     ctx = None
     if keep:
         ctx = dict(gctx)
@@ -759,56 +666,28 @@ def descriptor_forward(net, x, sn, keypoints, epoch, permute_idx, use_tc=True, k
 def _group_net_backward(bw, net, ctx, GY5):
     """Backward of _group_net_forward from GY5 [G, C5], the gradient of conv5's raw output rows (parameter gradients are
     accumulated into bw.grads; points / centres carry no gradient)."""
-    dev = bw.dev
-    Bp, M, K, D = ctx["Bp"], ctx["M"], ctx["K"], ctx["D"]
-    Q, G = Bp * M, Bp * M * K
-    lib, check, p, s = bw.lib, bw.check, ops._p, ops._stream
-    c1, c2, c3, c4, c5 = net.conv1, net.conv2, net.conv3, net.conv4, net.conv5
-    grp3 = ctx["grp3"]
-    C5 = c5.conv.weight.shape[0]
-    W5 = _w2d(c5.conv.weight)
-    bw.wgrad(GY5, ctx["Y4"], bw.g2d(c5.conv.weight), G, C5, W5.shape[1], prev=ctx["bn4"], name="wgrad_grp.conv5")
-    if getattr(c5, "norm", None) is None:
-        bw.colsum(GY5, bw.grads[c5.conv.bias], G, C5)          # a bias in front of a train-mode BN has exactly zero gradient
-    G_a4 = bw.dgrad(GY5, W5, G, name="dgrad_grp.conv5")
-    del GY5
-    GY4 = bw.bn_bwd(G_a4, ctx["Y4"], ctx["bn4"], c4.norm, G, G_a4.shape[1], name="bn_bwd_grp.conv4")
-    del G_a4
+    K, D = ctx["K"], ctx["D"]
+    L = ctx["layers"]                                                      # (conv_i, Y_i, bn_i), i = 1..4
+    c3, c4, bn3 = net.conv3, net.conv4, L[2][2]
+    GY4 = bw.layer_bwd(GY5, net.conv5, L[3], "grp.conv5", "bn_bwd_grp.conv4")
     # ---- conv4 on cat(y_first, broadcast max): Y4 = a3 WA^T + U[row/K] + b,  U = amax WB^T
     W4 = _w2d(c4.conv.weight)
     gW4 = bw.g2d(c4.conv.weight)
-    C4 = W4.shape[0]
-    bw.wgrad(GY4, ctx["Y3"], gW4[:, :D], G, C4, D, prev=ctx["bn3"], name="wgrad_grp.conv4")
-    G_a3 = bw.dgrad(GY4, _cols(W4, 0, D), G, name="dgrad_grp.conv4")                 # [G, D]
-    G_U = torch.empty((Q, C4), dtype=f32, device=dev)
-    check(lib.usip_group_sum(p(GY4), GY4.stride(0), p(G_U), G_U.stride(0), K, Q, C4, s()), "usip_group_sum")
+    bw.wgrad(GY4, L[2][1], gW4[:, :D], prev=bn3, name="wgrad_grp.conv4")
+    G_a3 = bw.dgrad(GY4, _cols(W4, 0, D), name="dgrad_grp.conv4")                   # [G, D]
+    G_U = ops.group_sum(GY4, K)                                                     # [Q, C4]
     del GY4
-    bw.wgrad(G_U, ctx["amax"], gW4[:, D:], Q, C4, D, name="wgrad_grp.conv4_node")
-    G_amax = bw.dgrad(G_U, _cols(W4, D), Q, name="dgrad_grp.conv4_node")             # [Q, D]
+    bw.wgrad(G_U, ctx["amax"], gW4[:, D:], name="wgrad_grp.conv4_node")
+    G_amax = bw.dgrad(G_U, _cols(W4, D), name="dgrad_grp.conv4_node")               # [Q, D]
     # the max path joins the dense gradient of a3 at the arg rows (the ReLU mask is applied by bn_bwd below)
-    gz = torch.empty((Q, D), dtype=f32, device=dev); arg3 = torch.empty((Q, D), dtype=i32, device=dev)
-    bn3 = ctx["bn3"]
-    check(lib.usip_groupmax_bwd_select(p(G_amax), G_amax.stride(0), p(grp3["gmax"]), p(grp3["gmin"]), p(grp3["amax"]),
-                                       p(grp3["amin"]), p(bn3.scale), p(bn3.shift), p(bn3.mean), p(bn3.invstd), p(gz), p(arg3),
-                                       None, Q, D, s()), "usip_groupmax_bwd_select")
-    check(lib.usip_groupmax_scatter_add(p(G_a3), G_a3.stride(0), p(G_amax), p(arg3), K, Q, D, s()), "usip_groupmax_scatter_add")
-    # ---- conv3, conv2, conv1
-    GY3 = bw.bn_bwd(G_a3, ctx["Y3"], bn3, c3.norm, G, D, name="bn_bwd_grp.conv3")
+    _, arg3, _ = bw.groupmax_select(G_amax, ctx["grp3"], bn3, False)
+    ops.groupmax_scatter_add(G_a3, G_amax, arg3, K)
+    # ---- conv3, conv2, then the weight gradient of conv1
+    GY = bw.bn_bwd(G_a3, L[2][1], bn3, c3.norm, name="bn_bwd_grp.conv3")
     del G_a3
-    W3 = _w2d(c3.conv.weight)
-    bw.wgrad(GY3, ctx["Y2"], bw.g2d(c3.conv.weight), G, W3.shape[0], W3.shape[1], prev=ctx["bn2"], name="wgrad_grp.conv3")
-    G_a2 = bw.dgrad(GY3, W3, G, name="dgrad_grp.conv3")
-    del GY3
-    GY2 = bw.bn_bwd(G_a2, ctx["Y2"], ctx["bn2"], c2.norm, G, G_a2.shape[1], name="bn_bwd_grp.conv2")
-    del G_a2
-    W2 = _w2d(c2.conv.weight)
-    bw.wgrad(GY2, ctx["Y1"], bw.g2d(c2.conv.weight), G, W2.shape[0], W2.shape[1], prev=ctx["bn1"], name="wgrad_grp.conv2")
-    G_a1 = bw.dgrad(GY2, W2, G, name="dgrad_grp.conv2")
-    del GY2
-    GY1 = bw.bn_bwd(G_a1, ctx["Y1"], ctx["bn1"], c1.norm, G, G_a1.shape[1], name="bn_bwd_grp.conv1")
-    del G_a1
-    W1 = _w2d(c1.conv.weight)
-    bw.wgrad(GY1, ctx["rows"], bw.g2d(c1.conv.weight), G, W1.shape[0], W1.shape[1], name="wgrad_grp.conv1")
+    for li in (2, 1):
+        GY = bw.layer_bwd(GY, L[li][0], L[li - 1], "grp.conv%d" % (li + 1), "bn_bwd_grp.conv%d" % li)
+    bw.wgrad(GY, ctx["rows"], bw.g2d(net.conv1.conv.weight), name="wgrad_grp.conv1")
 
 
 def descriptor_backward(net, ctx, g_desc):
@@ -818,16 +697,12 @@ def descriptor_backward(net, ctx, g_desc):
     a3 = relu(bn3(conv3(a2))), a2 = relu(bn2(conv2(a1))), a1 = relu(bn1(conv1(rows)))      (networks.py:375-383)."""
     dev = g_desc.device
     Bp, M, K, D = ctx["Bp"], ctx["M"], ctx["K"], ctx["D"]
-    Q, G = Bp * M, Bp * M * K
     bw = _Bwd(net, dev, ctx["use_tc"])
-    lib, check, p, s = bw.lib, bw.check, ops._p, ops._stream
     grp5 = ctx["grp5"]
     # ---- l2 normalisation and the max over the ball (conv5 is linear: the max of the raw output routes to its arg row)
-    G_y = torch.empty((Q, D), dtype=f32, device=dev)
-    check(lib.usip_l2norm_bwd(p(g_desc.contiguous()), p(grp5["gmax"]), grp5["gmax"].stride(0), p(G_y), G_y.stride(0), Bp, M, D, s()),
-          "usip_l2norm_bwd")
-    GY5 = torch.zeros((G, D), dtype=f32, device=dev)
-    check(lib.usip_groupmax_scatter_add(p(GY5), GY5.stride(0), p(G_y), p(grp5["amax"]), K, Q, D, s()), "usip_groupmax_scatter_add")
+    G_y = ops.l2norm_bwd(g_desc, grp5["gmax"], Bp, M)                       # [Q, D]
+    GY5 = torch.zeros((Bp * M * K, D), dtype=f32, device=dev)
+    ops.groupmax_scatter_add(GY5, G_y, grp5["amax"], K)
     _group_net_backward(bw, net, ctx, GY5)
     # conv1..conv4 biases sit in front of a train-mode BatchNorm: exactly zero gradient (left zero-initialised)
     return bw.result(net)

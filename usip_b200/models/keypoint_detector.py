@@ -249,17 +249,17 @@ class ModelDetector():
         # ---- losses, backward: d loss / d keypoints, sigmas
         if getattr(self, "_one", None) is None or self._one.device != kp.device:
             self._one = torch.ones(1, dtype=torch.float32, device=kp.device)
-        g_kpt, g_dst, g_ss, g_sd = losses.chamfer_prob_bwd(saved, self._one)
+        g_kpt, g_dst, g_ss, g_sd = ops.chamfer_prob_bwd(*saved, self._one)
         g_kp = torch.empty_like(kp)
-        g_kp[:B] = losses.transform_bwd(g_kpt, R, scale)
+        g_kp[:B] = ops.transform_points_bwd(g_kpt, R, scale)
         g_kp[B:] = g_dst
         for half, (kps, pc, snn, d, arg, _) in zip((g_kp[:B], g_kp[B:]), sides):
             n = d.numel()
             g = self._one.expand(d.shape[0], d.shape[1]).contiguous() if not plane else None
             if plane:
-                gk = losses.point_on_surface_bwd(kps, pc, snn, arg, torch.full_like(d, alpha / n))
+                gk = ops.point_on_surface(kps, pc, snn, arg, torch.full_like(d, alpha / n))
             else:
-                gk, _ = losses.pairmin_bwd(kps, pc, d, arg, g, want_b=False, scale=alpha / n)
+                gk, _ = ops.pairwise_min_bwd(kps, pc, d, arg, g, want_b=False, scale=alpha / n)
             half += gk
         g_sig = torch.cat((g_ss, g_sd), dim=0)
         engine.detector_backward(net, ctx, g_kp, g_sig)

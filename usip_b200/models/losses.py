@@ -7,73 +7,25 @@
 The (B,3,M,N) / (B,M,N) temporaries of the reference are never built: one tiled pairwise-L2 arg-min kernel
 (usip_pairwise_min_f32) serves all three, the reductions and the backward passes are small fused kernels.
 """
-import ctypes
-
 import torch
 import torch.nn as nn
 
-from usip_b200 import _lib, ops
-from usip_b200.ops import _p, _stream
+from usip_b200 import ops
 
 
 # ---- functional cores: used by the autograd Functions below and by the autograd-free train step of ModelDetector ----
-def pairmin_bwd(a, b, d, arg, g, want_b=False, scale=1.0):
-    """Gradient of d_i = min_j ||a_i - b_j|| w.r.t. a (and b): g (B,Ma) upstream, times `scale`."""
-    B, _, Ma = a.shape
-    ga = torch.empty_like(a)
-    gb = torch.zeros_like(b) if want_b else None
-    _lib.check(_lib.load().usip_pairwise_min_bwd(_p(a), _p(b), _p(d), _p(arg), _p(g.contiguous()), float(scale), _p(ga),
-                                                 _p(gb), B, Ma, b.shape[2], _stream()), "usip_pairwise_min_bwd")
-    return ga, gb
-
-
 def chamfer_prob_fwd(src, dst, sig_src, sig_dst):
-    """ChamferLoss_Brute sigma branch (losses.py:79-97): -> (out3 = [loss, pure, weighted], saved)."""
+    """ChamferLoss_Brute sigma branch (losses.py:79-97): -> (out3 = [loss, pure, weighted], saved), where saved are the
+    leading arguments of ops.chamfer_prob_bwd."""
     d_sd, i_sd = ops.pairwise_min(src, dst)
     d_ds, i_ds = ops.pairwise_min(dst, src)
     out3 = ops.chamfer_prob_reduce(d_sd, i_sd, d_ds, i_ds, sig_src, sig_dst)
     return out3, (src, dst, sig_src, sig_dst, d_sd, i_sd, d_ds, i_ds)
 
 
-def chamfer_prob_bwd(saved, g_loss):
-    """-> (g_src, g_dst, g_sig_src, g_sig_dst) for the upstream gradient g_loss (1-element tensor) of the chamfer loss."""
-    src, dst, sig_src, sig_dst, d_sd, i_sd, d_ds, i_ds = saved
-    B, _, M = src.shape
-    N = dst.shape[2]
-    g_src = torch.zeros_like(src); g_dst = torch.zeros_like(dst)
-    g_ss = torch.zeros_like(sig_src); g_sd = torch.zeros_like(sig_dst)
-    gout = g_loss.reshape(1).to(torch.float32).contiguous()
-    _lib.check(_lib.load().usip_chamfer_prob_bwd(_p(src), _p(dst), _p(sig_src), _p(sig_dst), _p(d_sd), _p(i_sd),
-                                                 _p(d_ds), _p(i_ds), _p(gout), _p(g_src), _p(g_dst), _p(g_ss),
-                                                 _p(g_sd), B, M, N, _stream()), "usip_chamfer_prob_bwd")
-    return g_src, g_dst, g_ss, g_sd
-
-
-def transform_bwd(g, R, scale):
-    g = g.contiguous()
-    B, _, M = g.shape
-    gk = torch.empty_like(g)
-    _lib.check(_lib.load().usip_transform_points_bwd(_p(g), _p(R), _p(scale), _p(gk), B, M, _stream()),
-               "usip_transform_points_bwd")
-    return gk
-
-
 def point_on_surface_fwd(kp, pc, sn):
-    B, _, M = kp.shape
     _, arg = ops.pairwise_min(kp, pc)                       # nearest cloud point of every keypoint (not differentiated)
-    loss = torch.empty((B, M), dtype=torch.float32, device=kp.device)
-    _lib.check(_lib.load().usip_point_on_surface(_p(kp), _p(pc), _p(sn), _p(arg), None, _p(loss), None, B, M, pc.shape[2],
-                                                 sn.shape[1], _stream()), "usip_point_on_surface")
-    return loss, arg
-
-
-def point_on_surface_bwd(kp, pc, sn, arg, g):
-    B, _, M = kp.shape
-    g_kp = torch.empty_like(kp)
-    _lib.check(_lib.load().usip_point_on_surface(_p(kp), _p(pc), _p(sn), _p(arg), _p(g.reshape(B, M).contiguous().float()),
-                                                 None, _p(g_kp), B, M, pc.shape[2], sn.shape[1], _stream()),
-               "usip_point_on_surface")
-    return g_kp
+    return ops.point_on_surface(kp, pc, sn, arg), arg
 
 
 class _PairMinFn(torch.autograd.Function):
@@ -91,7 +43,7 @@ class _PairMinFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         a, b, d, arg = ctx.saved_tensors
-        ga, gb = pairmin_bwd(a, b, d, arg, g, want_b=ctx.needs_input_grad[1])
+        ga, gb = ops.pairwise_min_bwd(a, b, d, arg, g, want_b=ctx.needs_input_grad[1])
         return (ga if ctx.needs_input_grad[0] else None), gb
 
 
@@ -110,7 +62,7 @@ class _ChamferProbFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g_loss, g_pure, g_weighted):
-        return chamfer_prob_bwd(ctx.saved_tensors, g_loss)
+        return ops.chamfer_prob_bwd(*ctx.saved_tensors, g_loss.reshape(1).to(torch.float32).contiguous())
 
 
 class _TransformFn(torch.autograd.Function):
@@ -126,7 +78,7 @@ class _TransformFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         R, scale = ctx.saved_tensors
-        return transform_bwd(g, R, scale), None, None, None
+        return ops.transform_points_bwd(g, R, scale), None, None, None
 
 
 class _MeanScaleFn(torch.autograd.Function):
@@ -190,7 +142,7 @@ class _PointOnSurfaceFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         kp, pc, sn, arg = ctx.saved_tensors
-        return point_on_surface_bwd(kp, pc, sn, arg, g), None, None
+        return ops.point_on_surface(kp, pc, sn, arg, g.reshape(arg.shape).contiguous().float()), None, None
 
 
 class PointOnSurfaceLoss(nn.Module):
@@ -223,17 +175,10 @@ class _DescTripletFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, anc, pos, neg, sigmas, gamma, sigma_max):
-        lib = _lib.load()
         a = anc.contiguous(); p_ = pos.contiguous(); n_ = neg.contiguous(); sg = sigmas.contiguous().float()
-        B, C, M = a.shape
-        dev = a.device
-        dpos = torch.empty((B, M), dtype=torch.float32, device=dev); dneg = torch.empty_like(dpos)
-        ipos = torch.empty((B, M), dtype=torch.int32, device=dev); ineg = torch.empty_like(ipos)
-        _lib.check(lib.usip_desc_pairmin_f32(_p(a), _p(p_), _p(dpos), _p(ipos), B, C, M, p_.shape[2], _stream()), "usip_desc_pairmin_f32")
-        _lib.check(lib.usip_desc_pairmin_f32(_p(a), _p(n_), _p(dneg), _p(ineg), B, C, M, n_.shape[2], _stream()), "usip_desc_pairmin_f32")
-        loss = torch.empty_like(dpos); active = torch.empty((B,), dtype=torch.float32, device=dev)
-        _lib.check(lib.usip_desc_triplet(_p(dpos), _p(dneg), _p(sg), float(gamma), float(sigma_max), _p(loss), _p(active),
-                                         B, M, _stream()), "usip_desc_triplet")
+        dpos, ipos = ops.desc_pairmin(a, p_)
+        dneg, ineg = ops.desc_pairmin(a, n_)
+        loss, active = ops.desc_triplet(dpos, dneg, sg, gamma, sigma_max)
         ctx.save_for_backward(a, p_, n_, sg, dpos, ipos, dneg, ineg)
         ctx.gamma, ctx.sigma_max = float(gamma), float(sigma_max)
         ctx.mark_non_differentiable(active)
@@ -242,12 +187,8 @@ class _DescTripletFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_loss, g_active):
         a, p_, n_, sg, dpos, ipos, dneg, ineg = ctx.saved_tensors
-        B, C, M = a.shape
-        g_a = torch.zeros_like(a); g_p = torch.zeros_like(p_); g_n = torch.zeros_like(n_)
-        _lib.check(_lib.load().usip_desc_triplet_bwd(_p(a), _p(p_), _p(n_), _p(dpos), _p(ipos), _p(dneg), _p(ineg), _p(sg),
-                                                     ctx.gamma, ctx.sigma_max, _p(g_loss.contiguous().float()), _p(g_a), _p(g_p),
-                                                     _p(g_n), B, C, M, p_.shape[2], n_.shape[2], _stream()),
-                   "usip_desc_triplet_bwd")
+        g_a, g_p, g_n = ops.desc_triplet_bwd(a, p_, n_, dpos, ipos, dneg, ineg, sg, ctx.gamma, ctx.sigma_max,
+                                             g_loss.contiguous().float())
         return g_a, g_p, g_n, None, None, None
 
 

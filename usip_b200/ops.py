@@ -264,6 +264,11 @@ def layer_fwd(X, W, bias, P, Cin, Cout, ldx=None, ldw=None, in_scale=None, in_sh
           "usip_layer_fwd_tc" if (precision == 1 and not tc_packed) else "usip_layer_fwd")
 
 
+def layer_tc_pack_many(descs):
+    arr = (LayerDesc * len(descs))(*descs)
+    check(_lib.load().usip_layer_tc_pack_many(arr, len(descs), _stream()), "usip_layer_tc_pack_many")
+
+
 def bn_finalize(stat_partial, ntiles, count, C, gamma, beta, eps, momentum, running_mean, running_var,
                 scale, shift, save_mean=None, save_invstd=None):
     check(_lib.load().usip_bn_finalize(_p(stat_partial), ntiles, int(count), C, _p(gamma), _p(beta), float(eps),
@@ -295,6 +300,117 @@ def head_finalize(out4, cluster_mean, lb, B, M):
     return kp, sig
 
 
+def l2norm_to_bcm(X, B, M):
+    out = torch.empty((B, X.shape[1], M), dtype=f32, device=X.device)
+    check(_lib.load().usip_l2norm_to_bcm(_p(X), X.stride(0), _p(out), None, B, M, X.shape[1], _stream()), "usip_l2norm_to_bcm")
+    return out
+
+
+# ----------------------------------------------------------------------------- backward of the shared-MLP stack
+# G / GY are [rows, C] gradients; rows and channels come from their shapes.  "+=" marks outputs accumulated into.
+def head_bwd(g_kp, g_sig, out4, B, M):
+    G = torch.empty((B * M, 4), dtype=f32, device=out4.device)
+    check(_lib.load().usip_head_bwd(_p(g_kp), _p(g_sig), _p(out4), out4.stride(0), _p(G), B, M, _stream()), "usip_head_bwd")
+    return G
+
+
+def wgrad(GY, X, gW, in_scale=None, in_shift=None, in_relu=False, precision=0):
+    """gW [Cout, Cin] += GY^T act(X), act = the layer's prologue (folded BN affine, ReLU)."""
+    check(_lib.load().usip_wgrad(_p(GY), GY.stride(0), _p(X), X.stride(0), _p(in_scale), _p(in_shift), 1 if in_relu else 0,
+                                 _p(gW), gW.stride(0), GY.shape[0], gW.shape[0], gW.shape[1], precision, _stream()), "usip_wgrad")
+
+
+def colsum(G, out):
+    """out [C] += column sums of G."""
+    check(_lib.load().usip_colsum(_p(G), G.stride(0), _p(out), G.shape[0], G.shape[1], _stream()), "usip_colsum")
+
+
+def bn_bwd_reduce(G, Y, scale, shift, mean, invstd, relu):
+    P, C = G.shape
+    part = torch.empty(((P + 127) // 128, 2, C), dtype=f32, device=G.device)
+    check(_lib.load().usip_bn_bwd_reduce(_p(G), G.stride(0), _p(Y), Y.stride(0), _p(scale), _p(shift), _p(mean), _p(invstd),
+                                         1 if relu else 0, _p(part), P, C, _stream()), "usip_bn_bwd_reduce")
+    return part
+
+
+def bn_bwd_finalize(part, count, g_gamma, g_beta):
+    """g_gamma / g_beta += the BN parameter gradients over `count` rows; returns the constants (c1, c2) of bn_bwd_apply."""
+    ntiles, _, C = part.shape
+    c1 = torch.empty(C, dtype=f32, device=part.device); c2 = torch.empty(C, dtype=f32, device=part.device)
+    check(_lib.load().usip_bn_bwd_finalize(_p(part), ntiles, count, C, _p(g_gamma), _p(g_beta), _p(c1), _p(c2), 1, _stream()),
+          "usip_bn_bwd_finalize")
+    return c1, c2
+
+
+def bn_bwd_apply(G, Y, scale, shift, mean, invstd, c1, c2, relu):
+    P, C = G.shape
+    GY = torch.empty((P, C), dtype=f32, device=G.device)
+    check(_lib.load().usip_bn_bwd_apply(_p(G), G.stride(0), _p(Y), Y.stride(0), _p(scale), _p(shift), _p(mean), _p(invstd),
+                                        _p(c1), _p(c2), 1 if relu else 0, _p(GY), GY.stride(0), P, C, _stream()),
+          "usip_bn_bwd_apply")
+    return GY
+
+
+def groupmax_bwd_select(Gout, gmax, gmin, amax, amin, scale, shift, mean, invstd, with_stats):
+    """-> (gz, argsel[, BN-backward partial sums over the selected rows if with_stats, else None]), all [Q, C]-shaped."""
+    Q, C = Gout.shape
+    gz = torch.empty((Q, C), dtype=f32, device=Gout.device)
+    argsel = torch.empty((Q, C), dtype=i32, device=Gout.device)
+    part = torch.empty(((Q + 127) // 128, 2, C), dtype=f32, device=Gout.device) if with_stats else None
+    check(_lib.load().usip_groupmax_bwd_select(_p(Gout), Gout.stride(0), _p(gmax), _p(gmin), _p(amax), _p(amin), _p(scale),
+                                               _p(shift), _p(mean), _p(invstd), _p(gz), _p(argsel), _p(part), Q, C, _stream()),
+          "usip_groupmax_bwd_select")
+    return gz, argsel, part
+
+
+def groupmax_scatter_add(G, gsrc, argsel, K):
+    """G [Q*K, C]: row argsel[q, c] of group q, column c += gsrc[q, c]."""
+    Q, C = gsrc.shape
+    check(_lib.load().usip_groupmax_scatter_add(_p(G), G.stride(0), _p(gsrc), _p(argsel), K, Q, C, _stream()),
+          "usip_groupmax_scatter_add")
+
+
+def groupmax_bwd_apply(Y, gz, argsel, scale, mean, invstd, c1, c2, K):
+    P, C = Y.shape[0], gz.shape[1]
+    GY = torch.empty((P, C), dtype=f32, device=Y.device)
+    check(_lib.load().usip_groupmax_bwd_apply(_p(Y), Y.stride(0), _p(gz), _p(argsel), _p(scale), _p(mean), _p(invstd), _p(c1),
+                                              _p(c2), _p(GY), GY.stride(0), K, P, C, _stream()), "usip_groupmax_bwd_apply")
+    return GY
+
+
+def group_sum(G, K):
+    Q, C = G.shape[0] // K, G.shape[1]
+    out = torch.empty((Q, C), dtype=f32, device=G.device)
+    check(_lib.load().usip_group_sum(_p(G), G.stride(0), _p(out), out.stride(0), K, Q, C, _stream()), "usip_group_sum")
+    return out
+
+
+def seg_sum(G, seg_off, B, N, M):
+    out = torch.empty((B * M, G.shape[1]), dtype=f32, device=G.device)
+    check(_lib.load().usip_seg_sum(_p(G), G.stride(0), _p(seg_off), _p(out), out.stride(0), B, N, M, G.shape[1], _stream()),
+          "usip_seg_sum")
+    return out
+
+
+def unpool_scatter(G, gp, arg, accumulate):
+    """Backward of segmax: G[arg[q, c], c] = gp[q, c], or += with accumulate."""
+    check(_lib.load().usip_unpool_scatter(_p(G), G.stride(0), _p(gp), gp.stride(0), _p(arg), gp.shape[0], gp.shape[1],
+                                          1 if accumulate else 0, _stream()), "usip_unpool_scatter")
+
+
+def knn_combine_bwd(GY, pts, knn_idx, GZ, gW, B, M, K):
+    """Backward of knn_combine: GZ += GY scattered by neighbour, gW[:, 0:3] += GY^T delta_xyz."""
+    check(_lib.load().usip_knn_combine_bwd(_p(GY), GY.stride(0), _p(pts), _p(knn_idx), _p(GZ), GZ.stride(0), _p(gW),
+                                           gW.stride(0), B, M, K, GY.shape[1], _stream()), "usip_knn_combine_bwd")
+
+
+def l2norm_bwd(g, Y, B, M):
+    GY = torch.empty((B * M, Y.shape[1]), dtype=f32, device=Y.device)
+    check(_lib.load().usip_l2norm_bwd(_p(g.contiguous()), _p(Y), Y.stride(0), _p(GY), GY.stride(0), B, M, Y.shape[1],
+                                      _stream()), "usip_l2norm_bwd")
+    return GY
+
+
 # ----------------------------------------------------------------------------- losses
 # databases at least this large go through the cell grid (usip_pairwise_min_grid_f32); smaller ones stay brute force
 PAIRWISE_MIN_GRID_FROM = 4096
@@ -322,6 +438,16 @@ def pairwise_min(a, b, method="auto"):
     return d, arg
 
 
+def pairwise_min_bwd(a, b, d, arg, g, want_b=False, scale=1.0):
+    """Gradient of d_i = min_j ||a_i - b_j|| w.r.t. a (and b): g (B,Ma) upstream, times `scale` -> (ga, gb or None)."""
+    B, _, Ma = a.shape
+    ga = torch.empty_like(a)
+    gb = torch.zeros_like(b) if want_b else None
+    check(_lib.load().usip_pairwise_min_bwd(_p(a), _p(b), _p(d), _p(arg), _p(g.contiguous()), float(scale), _p(ga), _p(gb),
+                                            B, Ma, b.shape[2], _stream()), "usip_pairwise_min_bwd")
+    return ga, gb
+
+
 def chamfer_prob_reduce(d_sd, i_sd, d_ds, i_ds, sig_src, sig_dst):
     B, M = d_sd.shape
     N = d_ds.shape[1]
@@ -329,6 +455,17 @@ def chamfer_prob_reduce(d_sd, i_sd, d_ds, i_ds, sig_src, sig_dst):
     check(_lib.load().usip_chamfer_prob_reduce(_p(d_sd), _p(i_sd), _p(d_ds), _p(i_ds), _p(sig_src), _p(sig_dst),
                                                _p(out), B, M, N, _stream()), "usip_chamfer_prob_reduce")
     return out
+
+
+def chamfer_prob_bwd(src, dst, sig_src, sig_dst, d_sd, i_sd, d_ds, i_ds, gout):
+    B, _, M = src.shape
+    N = dst.shape[2]
+    g_src = torch.zeros_like(src); g_dst = torch.zeros_like(dst)
+    g_ss = torch.zeros_like(sig_src); g_sd = torch.zeros_like(sig_dst)
+    check(_lib.load().usip_chamfer_prob_bwd(_p(src), _p(dst), _p(sig_src), _p(sig_dst), _p(d_sd), _p(i_sd), _p(d_ds), _p(i_ds),
+                                            _p(gout), _p(g_src), _p(g_dst), _p(g_ss), _p(g_sd), B, M, N, _stream()),
+          "usip_chamfer_prob_bwd")
+    return g_src, g_dst, g_ss, g_sd
 
 
 def transform_points(kp, R, scale, shift):
@@ -339,7 +476,60 @@ def transform_points(kp, R, scale, shift):
     return out
 
 
+def transform_points_bwd(g, R, scale):
+    g = g.contiguous()
+    B, _, M = g.shape
+    gk = torch.empty_like(g)
+    check(_lib.load().usip_transform_points_bwd(_p(g), _p(R), _p(scale), _p(gk), B, M, _stream()), "usip_transform_points_bwd")
+    return gk
+
+
 def mean_scale(d, alpha):
     out = torch.empty((1,), dtype=f32, device=d.device)
     check(_lib.load().usip_mean_scale(_p(d), d.numel(), float(alpha), _p(out), _stream()), "usip_mean_scale")
     return out
+
+
+def point_on_surface(kp, pc, sn, arg, g=None):
+    """-> loss (B,M), or with the upstream gradient g (B,M) the gradient w.r.t. kp (B,3,M) instead."""
+    B, _, M = kp.shape
+    loss = torch.empty((B, M), dtype=f32, device=kp.device) if g is None else None
+    g_kp = None if g is None else torch.empty_like(kp)
+    check(_lib.load().usip_point_on_surface(_p(kp), _p(pc), _p(sn), _p(arg), _p(g), _p(loss), _p(g_kp), B, M, pc.shape[2],
+                                            sn.shape[1], _stream()), "usip_point_on_surface")
+    return loss if g is None else g_kp
+
+
+def desc_pairmin(a, b):
+    """a (B,C,Ma), b (B,C,Nb) -> (min_d (B,Ma) f32, arg (B,Ma) i32)."""
+    B, C, Ma = a.shape
+    d = torch.empty((B, Ma), dtype=f32, device=a.device)
+    arg = torch.empty((B, Ma), dtype=i32, device=a.device)
+    check(_lib.load().usip_desc_pairmin_f32(_p(a), _p(b), _p(d), _p(arg), B, C, Ma, b.shape[2], _stream()),
+          "usip_desc_pairmin_f32")
+    return d, arg
+
+
+def desc_triplet(dpos, dneg, sigma, gamma, sigma_max):
+    B, M = dpos.shape
+    loss = torch.empty_like(dpos)
+    active = torch.empty((B,), dtype=f32, device=dpos.device)
+    check(_lib.load().usip_desc_triplet(_p(dpos), _p(dneg), _p(sigma), float(gamma), float(sigma_max), _p(loss), _p(active),
+                                        B, M, _stream()), "usip_desc_triplet")
+    return loss, active
+
+
+def desc_triplet_bwd(anc, pos, neg, dpos, ipos, dneg, ineg, sigma, gamma, sigma_max, g_loss):
+    B, C, M = anc.shape
+    g_a = torch.zeros_like(anc); g_p = torch.zeros_like(pos); g_n = torch.zeros_like(neg)
+    check(_lib.load().usip_desc_triplet_bwd(_p(anc), _p(pos), _p(neg), _p(dpos), _p(ipos), _p(dneg), _p(ineg), _p(sigma),
+                                            float(gamma), float(sigma_max), _p(g_loss), _p(g_a), _p(g_p), _p(g_n), B, C, M,
+                                            pos.shape[2], neg.shape[2], _stream()), "usip_desc_triplet_bwd")
+    return g_a, g_p, g_n
+
+
+# ----------------------------------------------------------------------------- optimizer
+def adam_step(p, g, m, v, lr_dev, step_dev, arrive, beta1, beta2, eps, grad_scale):
+    with torch.cuda.device(p.device):
+        check(_lib.load().usip_adam_step(_p(p), _p(g), _p(m), _p(v), _p(lr_dev), _p(step_dev), _p(arrive), float(beta1),
+                                         float(beta2), float(eps), float(grad_scale), p.numel(), _stream()), "usip_adam_step")

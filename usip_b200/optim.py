@@ -14,11 +14,9 @@ same update is one kernel launch:
     (ModelDetector.optimize replays the whole train step as one graph); `param_groups[i]['lr']` stays the knob callers turn
     (ModelDetector.update_learning_rate), it is mirrored to the device when it changes.
 """
-import ctypes
-
 import torch
 
-from . import _lib
+from . import _lib, ops
 
 
 class FlatAdam(torch.optim.Optimizer):
@@ -99,12 +97,7 @@ class FlatAdam(torch.optim.Optimizer):
                     p.grad = p._usip_flat_grad
         g = self.param_groups[0]
         b1, b2 = g["betas"]
-        lib = _lib.load()
-        P = ctypes.c_void_p
-        with torch.cuda.device(self.flat_p.device):
-            _lib.check(lib.usip_adam_step(P(self.flat_p.data_ptr()), P(self.flat_g.data_ptr()), P(self.exp_avg.data_ptr()),
-                                          P(self.exp_avg_sq.data_ptr()), P(self.lr_dev.data_ptr()), P(self.step_dev.data_ptr()),
-                                          P(self._arrive.data_ptr()), float(b1), float(b2), float(g["eps"]), float(self.grad_scale),
-                                          self.n, ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)), "usip_adam_step")
+        ops.adam_step(self.flat_p, self.flat_g, self.exp_avg, self.exp_avg_sq, self.lr_dev, self.step_dev, self._arrive,
+                      b1, b2, g["eps"], self.grad_scale)
         _lib.WEIGHT_GEN[0] += 1                                 # the raw-pointer update does not bump autograd versions
         return None
