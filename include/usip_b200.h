@@ -322,6 +322,41 @@ int usip_wgrad(const float* GY, int ldg, const float* X, int ldx, const float* i
 int usip_adam_step(float* p, const float* g, float* m, float* v, const float* lr_dev, int64_t* step_dev, uint32_t* arrive,
                    float beta1, float beta2, float eps, float grad_scale, int64_t n, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 6. Registration evaluation       evaluation/matlab/eval_outdoor/{kitti,oxford}/evaluate_*.m, eval_outdoor/external/
+ * ---------------------------------------------------------------------------------------------- */
+/* pdist2(b', a', 'euclidean', 'smallest', k) (evaluate_kitti.m:53, evaluate_oxford.m:63,67): for every a column the k
+ * (1..8) nearest b columns in ascending distance, ties to the smaller index.  a (B,C,Ma), b (B,C,Mb) channel-major;
+ * na / nb (B) valid counts or NULL (all).  idx (B,Ma,k) i32, -1 past the valid queries or candidates; dist (B,Ma,k) f32
+ * or NULL.  Same arithmetic as usip_desc_pairmin_f32: the k = 1 column equals its arg bit for bit.  C <= 426. */
+int usip_desc_knn_f32(const float* a, const float* b, const int32_t* na, const int32_t* nb, int32_t* idx, float* dist,
+                      int B, int C, int Ma, int Mb, int k, void* stream);
+
+/* Correspondence list: the unique (anc, pos) rows of nn12 (B,Ma,k12) (anc i -> pos nn12[i]) and, if nn21 != NULL, of
+ * nn21 (B,Mb,k21) (pos j -> anc nn21[j]), in ascending (anc, pos) order -- union(matches12, matches21, 'rows') of
+ * evaluate_oxford.m:63-72; with nn21 NULL and k12 = 1, [i, nn(i)] in anc order (evaluate_kitti.m:53-54).  Entries
+ * outside [0, nb) / [0, na) are ignored.  corr (B,nmax,2) i32 (rows past count[b] are -1), count (B).
+ * Ma, Mb <= 1024; nmax >= min(Ma*k12 + Mb*k21, Ma*Mb). */
+int usip_corr_build(const int32_t* nn12, int k12, const int32_t* nn21, int k21, const int32_t* na, const int32_t* nb,
+                    int32_t* corr, int32_t* count, int B, int Ma, int Mb, int nmax, void* stream);
+
+/* Batched RANSAC rigid fit, ransacfitRt.m + ransac.m (s = 3, no degeneracy test, p, maxTrials) with the final
+ * least-squares refit of estimateRigidTransform.m.  Correspondence c of pair b: x = anc_xyz[b, corr[b,c,0]],
+ * y = pos_xyz[b, corr[b,c,1]] (f64 (B,Ma,3) / (B,Mb,3)), c < ncorr[b].  Inlier iff ||x - (R y + t)|| < threshold.
+ * Trial tau draws 3 distinct indices from Philox-4x32-10 keyed by (seed, b, tau), or reads samples (B,max_trials+1,3)
+ * when non-NULL; samples_out (same shape, or NULL) receives the indices of every trial scored.
+ * Out: Rt (B,3,4) f64 mapping pos-frame points into the anc frame (NaN when empty), n_inliers, trialcount, best_trial
+ * (-1 without a loop), inlier_mask (B,nmax) u8 = the best hypothesis's inliers (not recomputed after the refit),
+ * status 0 ok / 1 fewer than 3 correspondences / 2 fewer than 3 inliers.
+ * scratch: usip_ransac_rt_scratch_bytes(B, max_trials) bytes, 16-byte aligned.  12 launches: init, 5 x (score, scan)
+ * over a fixed chunk schedule of trials, refit; no host synchronisation. */
+size_t usip_ransac_rt_scratch_bytes(int B, int max_trials);
+int usip_ransac_rt(const double* anc_xyz, const double* pos_xyz, const int32_t* corr, const int32_t* ncorr,
+                   const int32_t* samples, int32_t* samples_out, double threshold, int max_trials, double p,
+                   unsigned long long seed, double* Rt, int32_t* n_inliers, int32_t* trialcount, int32_t* best_trial,
+                   uint8_t* inlier_mask, int32_t* status, void* scratch, size_t scratch_bytes, int B, int Ma, int Mb,
+                   int nmax, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -107,6 +107,12 @@ SIGNATURES = {
     "usip_head_bwd": (c_int, [c_ptr, c_ptr, c_ptr, c_int, c_ptr, c_int, c_int, c_ptr]),
     "usip_adam_step": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_f32, c_f32, c_f32, c_f32, c_i64, c_ptr]),
     "usip_wgrad": (c_int, [c_ptr, c_int, c_ptr, c_int, c_ptr, c_ptr, c_int, c_ptr, c_int, c_int, c_int, c_int, c_int, c_ptr]),
+    "usip_desc_knn_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_int, c_int, c_int, c_int, c_ptr]),
+    "usip_corr_build": (c_int, [c_ptr, c_int, c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_int, c_int, c_int, c_ptr]),
+    "usip_ransac_rt_scratch_bytes": (ctypes.c_size_t, [c_int, c_int]),
+    "usip_ransac_rt": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, ctypes.c_double, c_int, ctypes.c_double, ctypes.c_uint64,
+                               c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, ctypes.c_size_t, c_int, c_int, c_int, c_int,
+                               c_ptr]),
 }
 
 _lib = None
@@ -142,7 +148,8 @@ def load():
 WEIGHT_GEN = [0]
 
 # kernels launched per C-ABI call (for bench.py's gpu_launches claim); default 1
-KERNELS_PER_CALL = {"usip_cluster_sort": 3, "usip_pairwise_min_f32": 3, "usip_pairwise_min_grid_f32": 3, "usip_som_assign_grid_f32": 2, "usip_layer_fwd_tc": 2, "usip_ball_group_f32": 2}
+KERNELS_PER_CALL = {"usip_cluster_sort": 3, "usip_pairwise_min_f32": 3, "usip_pairwise_min_grid_f32": 3, "usip_som_assign_grid_f32": 2, "usip_layer_fwd_tc": 2, "usip_ball_group_f32": 2,
+                    "usip_ransac_rt": 12}
 LAUNCHES = [0]
 
 

@@ -10,9 +10,12 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_DIR = os.path.join(_HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libusip_b200.so")
-SOURCES = ["api.cu", "group.cu", "indexmax.cu", "ballquery.cu", "ballgroup.cu", "knngroup.cu", "loss.cu", "nngrid.cu", "mlp.cu", "mlp_tc.cu", "backward.cu", "wgrad_tc.cu", "fps.cu", "nms.cu", "optim.cu"]
+SOURCES = ["api.cu", "group.cu", "indexmax.cu", "ballquery.cu", "ballgroup.cu", "knngroup.cu", "loss.cu", "nngrid.cu", "mlp.cu", "mlp_tc.cu", "backward.cu", "wgrad_tc.cu", "fps.cu", "nms.cu", "optim.cu", "registration.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
+# per-source additions: the registration kernels evaluate one float64 rigid fit in two kernels and need the same bits in
+# both, so no multiply-add is contracted there
+SOURCE_FLAGS = {"registration.cu": ["-fmad=false"]}
 
 
 def _nvcc():
@@ -42,7 +45,7 @@ def build(force=False, verbose=False):
         src = os.path.join(CSRC, s)
         obj = os.path.join(objdir, s.replace(".cu", ".o"))
         if force or _stale(obj, [src] + headers):
-            cmd = [nvcc] + NVCC_FLAGS + os.environ.get("USIP_NVCC_EXTRA", "").split() + ["-c", src, "-o", obj]
+            cmd = [nvcc] + NVCC_FLAGS + SOURCE_FLAGS.get(s, []) + os.environ.get("USIP_NVCC_EXTRA", "").split() + ["-c", src, "-o", obj]
             if verbose:
                 print(" ".join(cmd))
             r = subprocess.run(cmd, capture_output=True, text=True)

@@ -2,6 +2,7 @@
 // Reference: models/losses.py:50-99 (ChamferLoss_Brute), :125-143 (SingleSideChamferLoss_Brute),
 // models/keypoint_detector.py:182-197.
 #include "common.cuh"
+#include "desc_dist.cuh"
 
 namespace usip {
 
@@ -300,13 +301,7 @@ desc_pairmin_kernel(const float* __restrict__ a, const float* __restrict__ b, fl
     for (int t = threadIdx.x; t < C * DP_J; t += 256) { int c = t / DP_J, j = t - c * DP_J; sb[t] = (j0 + j) < Nb ? pb[(size_t)c * Nb + j0 + j] : 0.f; }
     __syncthreads();
     float acc[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) acc[u] = 0.f;
-    for (int c = 0; c < C; ++c) {
-      const float av = sa[c * DP_Q + qi];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) { const float df = av - sb[c * DP_J + js * 8 + u]; acc[u] = fmaf(df, df, acc[u]); }
-    }
+    desc_sqdist_tile<8>(sa + qi, DP_Q, sb + js * 8, DP_J, C, acc);
 #pragma unroll
     for (int u = 0; u < 8; ++u) { const int j = j0 + js * 8 + u; if (j < Nb && acc[u] < best) { best = acc[u]; bj = j; } }
   }

@@ -533,3 +533,74 @@ def adam_step(p, g, m, v, lr_dev, step_dev, arrive, beta1, beta2, eps, grad_scal
     with torch.cuda.device(p.device):
         check(_lib.load().usip_adam_step(_p(p), _p(g), _p(m), _p(v), _p(lr_dev), _p(step_dev), _p(arrive), float(beta1),
                                          float(beta2), float(eps), float(grad_scale), p.numel(), _stream()), "usip_adam_step")
+
+
+# ----------------------------------------------------------------------------- registration evaluation
+def desc_knn(a, b, k, na=None, nb=None, want_dist=False):
+    """a (B,C,Ma), b (B,C,Mb) f32, na / nb (B) i32 valid counts or None -> idx (B,Ma,k) i32 (-1 where there is no
+    candidate) and, with want_dist, dist (B,Ma,k) f32: the k nearest b columns of every a column, ties to the smaller index."""
+    _req(a, f32, "a"); _req(b, f32, "b")
+    B, C, Ma = a.shape
+    Mb = b.shape[2]
+    idx = torch.empty((B, Ma, int(k)), dtype=i32, device=a.device)
+    dist = torch.empty((B, Ma, int(k)), dtype=f32, device=a.device) if want_dist else None
+    with torch.cuda.device(a.device):
+        check(_lib.load().usip_desc_knn_f32(_p(a), _p(b), _p(na), _p(nb), _p(idx), _p(dist), B, C, Ma, Mb, int(k), _stream()),
+              "usip_desc_knn_f32")
+    return (idx, dist) if want_dist else idx
+
+
+def corr_build(nn12, Mb, nn21=None, na=None, nb=None):
+    """nn12 (B,Ma,k12) i32 anc -> pos indices in [0, Mb), nn21 (B,Mb,k21) i32 pos -> anc or None -> (corr (B,nmax,2) i32,
+    count (B) i32): the unique (anc, pos) rows in ascending order (rows past count are -1)."""
+    _req(nn12, i32, "nn12")
+    B, Ma, k12 = nn12.shape
+    Mb, k21 = int(Mb), 0
+    if nn21 is not None:
+        _req(nn21, i32, "nn21")
+        if nn21.shape[:2] != (B, Mb):
+            raise RuntimeError("nn21: expected (%d, %d, k), got %s" % (B, Mb, tuple(nn21.shape)))
+        k21 = nn21.shape[2]
+    nmax = max(1, min(Ma * k12 + Mb * k21, Ma * Mb))
+    corr = torch.empty((B, nmax, 2), dtype=i32, device=nn12.device)
+    count = torch.empty((B,), dtype=i32, device=nn12.device)
+    with torch.cuda.device(nn12.device):
+        check(_lib.load().usip_corr_build(_p(nn12), k12, _p(nn21), k21, _p(na), _p(nb), _p(corr), _p(count), B, Ma, Mb, nmax,
+                                          _stream()), "usip_corr_build")
+    return corr, count
+
+
+def ransac_rt(anc_xyz, pos_xyz, corr, ncorr, threshold, max_trials, p, seed, samples=None, want_samples=False):
+    """Batched RANSAC rigid fit (include/usip_b200.h): anc_xyz (B,Ma,3), pos_xyz (B,Mb,3) f64, corr (B,nmax,2) i32, ncorr (B)
+    i32 -> dict of Rt (B,3,4) f64, n_inliers, trialcount, best_trial, status (B) i32, inlier_mask (B,nmax) u8 and, with
+    want_samples, samples (B,max_trials+1,3) i32 (-1 for trials never scored)."""
+    f64 = torch.float64
+    _req(anc_xyz, f64, "anc_xyz"); _req(pos_xyz, f64, "pos_xyz"); _req(corr, i32, "corr"); _req(ncorr, i32, "ncorr")
+    B, Ma, _ = anc_xyz.shape
+    Mb = pos_xyz.shape[1]
+    nmax = corr.shape[1]
+    T = int(max_trials) + 1
+    dev = anc_xyz.device
+    if samples is not None:
+        _req(samples, i32, "samples")
+        if tuple(samples.shape) != (B, T, 3):
+            raise RuntimeError("samples: expected shape %s, got %s" % ((B, T, 3), tuple(samples.shape)))
+        n = ncorr.view(B, 1, 1)
+        if bool((((samples < 0) | (samples >= n)) & (n > 3)).any()):
+            raise RuntimeError("samples: indices must lie in [0, ncorr)")
+    out = {"Rt": torch.empty((B, 3, 4), dtype=f64, device=dev),
+           "n_inliers": torch.empty((B,), dtype=i32, device=dev), "trialcount": torch.empty((B,), dtype=i32, device=dev),
+           "best_trial": torch.empty((B,), dtype=i32, device=dev), "status": torch.empty((B,), dtype=i32, device=dev),
+           "inlier_mask": torch.empty((B, nmax), dtype=torch.uint8, device=dev)}
+    s_out = torch.full((B, T, 3), -1, dtype=i32, device=dev) if want_samples else None
+    lib = _lib.load()
+    nbytes = int(lib.usip_ransac_rt_scratch_bytes(B, int(max_trials)))
+    scratch = torch.empty(((nbytes + 15) // 16, 2), dtype=f64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.usip_ransac_rt(_p(anc_xyz), _p(pos_xyz), _p(corr), _p(ncorr), _p(samples), _p(s_out), float(threshold),
+                                 int(max_trials), float(p), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(out["Rt"]), _p(out["n_inliers"]),
+                                 _p(out["trialcount"]), _p(out["best_trial"]), _p(out["inlier_mask"]), _p(out["status"]),
+                                 _p(scratch), scratch.numel() * 8, B, Ma, Mb, nmax, _stream()), "usip_ransac_rt")
+    if want_samples:
+        out["samples"] = s_out
+    return out
